@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- thermo grid-points/s and achieved HBM GB/s vs roofline (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input.  Default workload (N=1) is
 BASELINE.json configs[1]: the fused thermo suite (t,q,p -> theta, es, rh, td, Tv) on IFS O1280
@@ -75,6 +75,7 @@ DEFAULT_WORKLOAD = "suite_tqp_o1280x137_f64"
 
 L2_FLUSH_BYTES = 384 << 20  # rotate small workloads over at least this many bytes (3 x the 126 MB L2)
 HBM_BUDGET_BYTES = 150e9    # resident arrays per GPU (of 180 GB): a shard larger than this is capped and reported so
+DUMP_BYTES = 64 << 20       # --dump-outputs writes at most this much in all
 
 # output name -> the public reference function it equals, on module m (the reference's earthkit.meteo.thermo or the
 # oracle, which mirrors its names): this is how a user of the reference computes the same fields
@@ -186,6 +187,7 @@ def build_step(kind, outputs, arrays, hyb=None):
             fn(a, b, c, outputs=outputs, out=o)
 
         step.n_sets = n_sets
+        step.last_out = lambda: sets[(state["i"] - 1) % n_sets][3]
         return step, bpp, out
     # ept + wet-bulb potential temperature ("direct"), BASELINE.json configs[2]: the two-output kernel
     from ctypes import c_int, c_int64, c_void_p
@@ -297,6 +299,24 @@ def parity_sample(kind, outputs, arrays, hyb, out, npl, dtype, n_target=1 << 20)
             res["n_nan"] += po["n_nan"]
     res["ok"] = bool(res["n_over_limit"] == 0 and res["nan_mismatches"] == 0 and res["inf_mismatches"] == 0)
     return res
+
+
+def dump_outputs(path, out, seed=0):
+    """Every output of one step as <path>/<name>.npy (flat, in the working dtype): all points when the outputs fit in
+    DUMP_BYTES, else the same sample of points for every output, drawn from `seed` and fixed by the field size, the dtype and
+    the number of outputs -- so two builds of the project run with the same arguments can be compared output for output."""
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    first = next(iter(out.values()))
+    n = first.numel()
+    k = min(n, (DUMP_BYTES - (64 << 10)) // (first.element_size() * len(out)))  # 64 KB left for the .npy headers
+    idx = None
+    if k < n:
+        idx = torch.from_numpy(np.sort(np.random.default_rng(seed).choice(n, k, replace=False))).to(first.device)
+    for name, x in out.items():
+        x = x.reshape(-1)
+        np.save(os.path.join(path, f"{name}.npy"), (x if idx is None else x[idx]).cpu().numpy())
 
 
 # --------------------------------------------------------------------------------------------------
@@ -505,6 +525,8 @@ def run_ours(args, wl):
 
     # ---- parity of the timed buffers (rank 0's field; every rank's for the sharded workload through the shard check)
     parity = parity_sample(kind, outputs, arrays, hyb, out, npl, dtype) if (rank == 0 and not args.no_parity) else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step.last_out() if hasattr(step, "last_out") else out)
 
     # ---- cross-shard check (SURVEY.md 8(e)): probe slabs of every shard are recomputed on rank 0 from the same seed
     shard_check = None
@@ -678,7 +700,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer legs")
     ap.add_argument("--no-e2e-pageable", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle check of the timed buffers")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) to DIR/<name>.npy, "
+                    "at most 64 MB in all: a fixed seeded sample of points when the whole outputs are larger")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the device path (--impl ours)")
     wl = dict(WORKLOADS[args.workload])
     if args.levels:
         wl["levels"] = args.levels

@@ -10,9 +10,12 @@ oracle/refshim.  Produces, next to this file:
                     re-packed column by column as float64 (keys "<file stem>/<column>").
 * ref_live.npz   -- inputs and outputs of the unmodified reference functions for every Case of
                     tests/cases.py on four input sets (seeded random, edge values, the reference's
-                    t_hum_p_data.csv grid, the moist-adiabat grid), float64 and float32.
+                    t_hum_p_data.csv grid, the moist-adiabat grid), float64 and float32.  The outputs on the
+                    seeded random set are in ref_live_rand_float64.npz and ref_live_rand_float32.npz.
 * ref_hybrid.npz -- hybrid-level pressure: the reference's golden vectors (tests/vertical/_hybrid_core_data.py) and live
-                    outputs of earthkit.meteo.vertical.pressure_on_hybrid_levels (SURVEY.md 8(f)-1).
+                    outputs of earthkit.meteo.vertical.pressure_on_hybrid_levels (SURVEY.md 8(f)-1); the live
+                    geopotential outputs (SURVEY.md 8(f)-2) are in ref_hybrid_geo.npz.
+  A set split over several files is merged back by tests/conftest.py; the split keeps every file under 1 MB.
 * ref_wind.npz   -- live outputs of the reference's elementwise wind functions (SURVEY.md 8(f)-3).
 * ifs_l137_ab.npz -- the IFS L137 A/B half-level coefficients from the reference's conf JSON (bench input layout).
 * PINNING.json   -- oracle-vs-reference comparison made at generation time (max relative
@@ -278,12 +281,20 @@ def pack_wind():
     return blob, mism
 
 
+def save_split(stem, blob, parts):
+    """`blob` as <stem>_<suffix>.npz for every (suffix, key prefix) of `parts` and <stem>.npz for the other keys."""
+    prefixes = tuple(pre for _, pre in parts)
+    np.savez_compressed(os.path.join(HERE, f"{stem}.npz"), **{k: v for k, v in blob.items() if not k.startswith(prefixes)})
+    for suffix, pre in parts:
+        np.savez_compressed(os.path.join(HERE, f"{stem}_{suffix}.npz"), **{k: v for k, v in blob.items() if k.startswith(pre)})
+
+
 def main():
     np.savez_compressed(os.path.join(HERE, "ref_csv.npz"), **pack_csvs())
     wind_blob, wind_mismatch = pack_wind()
     np.savez_compressed(os.path.join(HERE, "ref_wind.npz"), **wind_blob)
     hyb, hyb_mismatch = pack_hybrid()
-    np.savez_compressed(os.path.join(HERE, "ref_hybrid.npz"), **hyb)
+    save_split("ref_hybrid", hyb, [("geo", "geo/")])
     np.savez_compressed(os.path.join(HERE, "ifs_l137_ab.npz"), **pack_ifs_levels())
 
     sets = input_sets()
@@ -322,7 +333,7 @@ def main():
     pin["summary"] = {"worst_max_rel": worst, "nan_or_inf_mismatches": nan_mismatch, "n_entries": n_entries}
     pin["wind"] = {"arrays_not_bit_identical_to_reference": wind_mismatch, "n_arrays": sum(k.startswith("out/") for k in wind_blob)}
     pin["hybrid"] = {"arrays_not_bit_identical_to_reference": hyb_mismatch, "n_arrays": sum(k.startswith("live/float") or k.startswith("geo/float") for k in hyb)}
-    np.savez_compressed(os.path.join(HERE, "ref_live.npz"), **blob)
+    save_split("ref_live", blob, [("rand_float64", "out/rand/float64/"), ("rand_float32", "out/rand/float32/")])
     with open(os.path.join(HERE, "PINNING.json"), "w") as f:
         json.dump(pin, f, indent=1, sort_keys=True)
     print(json.dumps(pin["summary"]))

@@ -33,6 +33,23 @@ def test_other_ranks_of_the_reference_arm_exit_without_work():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_writes_all_points_or_a_fixed_sample(tmp_path, monkeypatch):
+    import bench
+
+    n = 50_000
+    out = {"theta": torch.arange(n, dtype=torch.float64), "rh": -torch.arange(n, dtype=torch.float32)}
+    bench.dump_outputs(str(tmp_path / "all"), out)
+    assert np.array_equal(np.load(tmp_path / "all" / "theta.npy"), out["theta"].numpy())
+    assert np.load(tmp_path / "all" / "rh.npy").dtype == np.float32
+    monkeypatch.setattr(bench, "DUMP_BYTES", (64 << 10) + 8 * 2 * 1000)  # room for 1000 points of each output
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), out)
+    theta, rh = np.load(tmp_path / "a" / "theta.npy"), np.load(tmp_path / "a" / "rh.npy")
+    assert theta.size == rh.size == 1000 and theta.dtype == np.float64 and rh.dtype == np.float32
+    assert np.all(np.diff(theta) > 0) and np.array_equal(rh, -theta.astype(np.float32))  # distinct points, the same for every output
+    assert np.array_equal(np.load(tmp_path / "b" / "theta.npy"), theta)  # and the same from run to run
+
+
 def test_workload_table_and_generator():
     import bench
     from synthetic import IfsField, sample_levels

@@ -16,12 +16,6 @@ OUTS = ("full", "half", "delta", "alpha")
 LEVEL_SETS = {"all": None, "lower": list(range(90, 138)), "reversed": list(range(137, 90, -1)), "two": [2, 1], "top": [1]}
 
 
-@pytest.fixture(scope="module")
-def hyb():
-    with np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_hybrid.npz")) as z:
-        return {k: z[k] for k in z.files}
-
-
 def _tol(name, f32):
     # delta/alpha difference quotients lose digits where ph1 - ph0 << ph0 (thin top layers); float32 as the reference's
     # own tolerance table (tests/vertical/test_array_vertical.py:196-203)

@@ -15,14 +15,6 @@ LEVEL_SETS = {"all": None, "lower": list(range(90, 138)), "reversed": list(range
 OUTS = ("full", "half", "delta", "alpha")
 
 
-@pytest.fixture(scope="module")
-def hyb():
-    import os
-
-    with np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_hybrid.npz")) as z:
-        return {k: z[k] for k in z.files}
-
-
 def test_oracle_matches_reference_golden_vectors(hyb):
     """tests/vertical/_hybrid_core_data.py, with the reference test's tolerances (atol 1e-8, rtol 1e-6; TT vertical :159-215)."""
     res = voracle.pressure_on_hybrid_levels(hyb["gold/A"], hyb["gold/B"], hyb["gold/p_surf"], output=list(OUTS))
