@@ -22,42 +22,23 @@ using namespace ek;
 #define EK_FAST_NS exactm
 #endif
 
-// levels whose t/q loads are in flight per thread.  Measured on B200 (O1280 x 137, fp64): 2 -> 10.3-11.0 ms,
-// 3 -> 12.0 ms, 4 -> 13.9 ms (register pressure at the 64-register cap), so 2.
-#ifndef EK_HYB_LU
-#define EK_HYB_LU 3
-#endif
-#ifndef EK_HYB_PREFETCH
-#define EK_HYB_PREFETCH 1  // L2 prefetch of a later level pair (EK_HYB_PF_DIST pairs ahead).  ncu on the round-1 kernel: 7.4 warps
-                           // per issue slot waiting on global loads, DRAM at 79 % -- the level loop keeps too few bytes in flight
-#endif
-#ifndef EK_HYB_PF_DIST
-#define EK_HYB_PF_DIST 2  // measured: 2 pairs ahead 0.86 vs 0.83 (hybrid suite), geometric height 0.91 vs 0.88
-#endif
-#ifndef EK_COL_PREFETCH
-#define EK_COL_PREFETCH 1  // the same for the column (geopotential) kernel
-#endif
-#ifndef EK_COL_PF_DIST
-#define EK_COL_PF_DIST 2
-#endif
-#ifndef EK_COL_LU
-#define EK_COL_LU 2  // levels in flight in the column (geopotential) kernel; measured 2 -> 4.46 ms, 4 -> 5.40 ms, 6 -> 7.68 ms
-                     // (O1280 x 137 fp64: beyond 2 the 64-register cap spills)
-#endif
-
-// Resident CTAs per SM the register budget of the two level-loop kernels is sized for.  Measured on B200 (O1280 x 137 fp64,
-// profiles/r02_ab_hybrid.log, with the L2 prefetch on): 3 CTAs (80 registers, no spills of the column state) beat 4 (64) for
-// the hybrid suite (0.70 -> 0.86 of the roofline) and the thickness / geopotential forms (0.885 -> 0.926); the geometric-height
-// forms keep 4 (0.877 vs 0.825 with 3).
-#ifndef EK_HYBS_MIN_CTAS
-#define EK_HYBS_MIN_CTAS 2  // with three levels in flight (EK_HYB_LU): 0.87 stable, against 0.80-0.88 for 3 CTAs x 2 levels
-#endif
-#ifndef EK_COL_MIN_CTAS
-#define EK_COL_MIN_CTAS 3
-#endif
-#ifndef EK_COL_MIN_CTAS_GEOM
-#define EK_COL_MIN_CTAS_GEOM 4
-#endif
+// The level loops of the hybrid suite and the column (geopotential) kernel issue the loads of several levels before any math
+// and ask L2 for a later group of levels while the current one is computed.  ncu on the round-1 hybrid suite, without the L2
+// prefetch: 7.4 warps per issue slot waiting on global loads, DRAM at 79 % -- the level loop kept too few bytes in flight.
+// Measured on B200, O1280 x 137 fp64 (profiles/r02_ab_hybrid.log, r02_ab_hybrid2.log, r02_ab_hybrid3.log):
+//   hybrid suite: 3 levels in flight at 2 CTAs per SM (128 registers) 0.87 of the roofline, stable; 3 levels at 3 CTAs spill
+//     (0.72), 4 levels at 2 CTAs 0.84, 2 levels at 3 CTAs 0.80-0.88;
+//   column kernel: 2 levels in flight 4.46 ms, 4 -> 5.40 ms, 6 -> 7.68 ms (at the 64-register cap: beyond 2 it spills); 3 CTAs (80
+//     registers, no spills of the column state) beat 4 (64) for the thickness / geopotential forms (0.885 -> 0.926), the
+//     geometric-height forms keep 4 (0.877 vs 0.825 with 3);
+//   prefetch distance: 2 groups of levels ahead 0.86 vs 0.83 (hybrid suite), geometric height 0.91 vs 0.88.
+constexpr int kHybLevels = 3;       // hybrid suite: levels whose t/q loads are in flight per thread
+constexpr int kHybMinCtas = 2;      // hybrid suite: resident CTAs per SM its register budget is sized for
+constexpr int kHybPfDist = 2;       // hybrid suite: groups of kHybLevels levels the L2 prefetch runs ahead
+constexpr int kColLevels = 2;       // column kernel, computed alpha/delta: levels in flight per thread (see CLU)
+constexpr int kColMinCtas = 3;      // column kernel: resident CTAs per SM
+constexpr int kColMinCtasGeom = 4;  // column kernel, geometric-height forms: resident CTAs per SM
+constexpr int kColPfDist = 2;       // column kernel: groups of levels the L2 prefetch runs ahead
 
 namespace {
 
@@ -148,7 +129,7 @@ struct HybridArgs {
 };
 
 template <typename T, bool VECOK>
-__global__ void __launch_bounds__(kThreads, EK_MIN_CTAS) hybrid_pressure_kernel(const HybridArgs g) {
+__global__ void __launch_bounds__(kThreads, kMinCtas) hybrid_pressure_kernel(const HybridArgs g) {
     constexpr int VEC = Vec16<T>::N;
     constexpr int TILE = kThreads * VEC;
     const bool want_da = g.delta != nullptr || g.alpha != nullptr;
@@ -237,10 +218,10 @@ template <typename T> __device__ __forceinline__ void coef_smem_fill(const T* A,
 template <typename T> constexpr unsigned coef_smem_bytes(int nhalf) { return 2u * (unsigned)nhalf * (unsigned)sizeof(T); }
 
 template <class Op, class OpE, typename T, bool VECOK>
-__global__ void __launch_bounds__(kThreads, EK_HYBS_MIN_CTAS) suite_hybrid_kernel(const SuiteHybridArgs g, const Params P) {
+__global__ void __launch_bounds__(kThreads, kHybMinCtas) suite_hybrid_kernel(const SuiteHybridArgs g, const Params P) {
     constexpr int VEC = Vec16<T>::N;
     constexpr int TILE = kThreads * VEC;
-    constexpr int LU = EK_HYB_LU;  // levels in flight per thread (their loads are issued before any math)
+    constexpr int LU = kHybLevels;  // levels in flight per thread (their loads are issued before any math)
 #if EK_LEAN_DEVICE
     if (sizeof(T) == 8) lean::init_tables();
 #endif
@@ -273,14 +254,12 @@ __global__ void __launch_bounds__(kThreads, EK_HYBS_MIN_CTAS) suite_hybrid_kerne
 #pragma unroll
                     for (int c = 0; c < 2; ++c) ld_row<T, VECOK>(tq[c] + (int64_t)(k + u) * g.npl, i0, g.npl, x[u][c], true);
                 }
-#if EK_HYB_PREFETCH
 #pragma unroll
-            for (int u = 0; u < LU; ++u)  // ask L2 for a later pair of levels while this pair is being computed
-                if (k + LU * EK_HYB_PF_DIST + u < k1) {
+            for (int u = 0; u < LU; ++u)  // ask L2 for a later group of levels while this group is being computed
+                if (k + LU * kHybPfDist + u < k1) {
 #pragma unroll
-                    for (int c = 0; c < 2; ++c) asm volatile("prefetch.global.L2 [%0];" ::"l"(tq[c] + (int64_t)(k + LU * EK_HYB_PF_DIST + u) * g.npl + i0));
+                    for (int c = 0; c < 2; ++c) asm volatile("prefetch.global.L2 [%0];" ::"l"(tq[c] + (int64_t)(k + LU * kHybPfDist + u) * g.npl + i0));
                 }
-#endif
 #pragma unroll
             for (int u = 0; u < LU; ++u) {
                 if (k + u >= k1) break;
@@ -331,14 +310,14 @@ struct GeoArgs {
 // MODE >= 0: the output form is a compile-time constant (the registers of zs / geom(zs) and the form choices drop out of
 // the level loop where they are not needed); MODE = -1: taken from g.mode at run time (the rarer launch shapes).
 template <typename T, bool GIVEN_AD, bool VECOK, int MODE>
-__global__ void __launch_bounds__(kThreads, (MODE >= EK_HM_GEOM_SEA ? EK_COL_MIN_CTAS_GEOM : EK_COL_MIN_CTAS)) column_geopotential_kernel(const GeoArgs g) {
+__global__ void __launch_bounds__(kThreads, (MODE >= EK_HM_GEOM_SEA ? kColMinCtasGeom : kColMinCtas)) column_geopotential_kernel(const GeoArgs g) {
     const int mode = MODE >= 0 ? MODE : g.mode;
     constexpr int VEC = Vec16<T>::N;
     constexpr int TILE = kThreads * VEC;
     constexpr int NARR = GIVEN_AD ? 4 : 2;
     // levels in flight per thread: the geometric-height forms (a reciprocal more per level) fit their registers only with one
     // (measured: geometric height 0.58 -> 0.61 with 1, thickness 0.77 -> 0.75)
-    constexpr int CLU = GIVEN_AD ? 2 : (MODE >= EK_HM_GEOM_SEA ? 1 : EK_COL_LU);
+    constexpr int CLU = GIVEN_AD ? 2 : (MODE >= EK_HM_GEOM_SEA ? 1 : kColLevels);
 #if EK_LEAN_DEVICE
     if (sizeof(T) == 8) lean::init_tables();
 #endif
@@ -381,14 +360,12 @@ __global__ void __launch_bounds__(kThreads, (MODE >= EK_HM_GEOM_SEA ? EK_COL_MIN
 #pragma unroll
                     for (int c = 0; c < NARR; ++c) ld_row<T, VECOK>(arr[c] + (int64_t)(k - u) * g.npl, i0, g.npl, x[u][c], true);
                 }
-#if EK_COL_PREFETCH
 #pragma unroll
             for (int u = 0; u < CLU; ++u)
-                if (k - CLU * EK_COL_PF_DIST - u >= 0) {
+                if (k - CLU * kColPfDist - u >= 0) {
 #pragma unroll
-                    for (int c = 0; c < NARR; ++c) asm volatile("prefetch.global.L2 [%0];" ::"l"(arr[c] + (int64_t)(k - CLU * EK_COL_PF_DIST - u) * g.npl + i0));
+                    for (int c = 0; c < NARR; ++c) asm volatile("prefetch.global.L2 [%0];" ::"l"(arr[c] + (int64_t)(k - CLU * kColPfDist - u) * g.npl + i0));
                 }
-#endif
 #pragma unroll
             for (int u = 0; u < CLU; ++u) {
                 const int kk = k - u;

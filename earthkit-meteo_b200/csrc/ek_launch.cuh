@@ -9,10 +9,6 @@
 
 #define EK_EXPORT __attribute__((visibility("default")))
 
-#ifndef EK_SMALL_WAVE_SPARE
-#define EK_SMALL_WAVE_SPARE 0  // CTA slots per SM a small-field launch leaves free for its successor in the stream (EK_PDL)
-#endif
-
 namespace ek {
 
 // defined in ek_api.cu
@@ -26,7 +22,7 @@ inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 // Dynamic shared memory of a launch: the lean float64 tables; float32 kernels use none.
 template <typename T> constexpr unsigned smem_for() { return sizeof(T) == 8 ? kSmemBytes : 0u; }
 
-// Once per kernel instantiation and device: ask for a shared-memory carve-out that holds EK_MIN_CTAS CTAs' tables, so the
+// Once per kernel instantiation and device: ask for a shared-memory carve-out that holds kMinCtas CTAs' tables, so the
 // tables never lower the occupancy the register budget was chosen for (the driver's default carve-out heuristic may
 // pick a smaller one).  `Kernel` is the address of the __global__ instantiation.
 template <auto Kernel> inline void prepare_smem(unsigned smem_bytes) {
@@ -36,7 +32,7 @@ template <auto Kernel> inline void prepare_smem(unsigned smem_bytes) {
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0) return;
     const uint64_t bit = dev < 64 ? (1ull << dev) : 0;
     if (bit && (done.load(std::memory_order_relaxed) & bit)) return;
-    const unsigned want = EK_MIN_CTAS * (smem_bytes + 1024u);  // + the per-CTA reservation
+    const unsigned want = kMinCtas * (smem_bytes + 1024u);  // + the per-CTA reservation
     int pct = (int)((want * 100u + 228u * 1024u - 1u) / (228u * 1024u));
     if (pct > 100) pct = 100;
     cudaFuncSetAttribute(Kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
@@ -68,7 +64,7 @@ inline void launch_streaming(unsigned blocks, unsigned smem, cudaStream_t st, Ar
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = EK_PDL ? 1 : 0;
+    cfg.numAttrs = 1;
     cudaLaunchKernelEx(&cfg, Kernel, args...);
 }
 
@@ -114,7 +110,7 @@ int launch(const char* what, const ek_operand* ins, void* const* outs, int64_t n
     // small fields (a few tiles per resident CTA, e.g. one ERA5 level): exactly one resident wave -- every CTA copies the lean
     // tables once and walks its 2-3 tiles back to back instead of a second, partial wave of CTAs queueing behind the first
     // (theta + rh on 1 M points, graph replay: 14.4 -> 12.3 us; profiles/r02_kbench_era5_ctas.log)
-    const int64_t wave = (int64_t)sms * (MinCtasOf<Op>::value - EK_SMALL_WAVE_SPARE);
+    const int64_t wave = (int64_t)sms * MinCtasOf<Op>::value;
     if (ntiles <= 8 * wave && wave < cap) cap = wave;
     int64_t blocks = ntiles > tail_blocks ? ntiles : tail_blocks;
     if (blocks > cap) blocks = cap;

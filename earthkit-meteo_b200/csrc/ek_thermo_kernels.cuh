@@ -3,7 +3,7 @@
 // The path is elementwise with no reuse, so the design is the HBM-streaming one (SURVEY.md §8(d)):
 //   * 128-bit coalesced loads/stores (double2 / float4) with streaming cache hints (ld.global.cs /
 //     st.global.cs: the data is touched once, keep it out of the way in L1/L2);
-//   * each thread front-loads EK_UNROLL vectors per input before any math so that enough bytes are in
+//   * each thread front-loads kUnroll vectors per input before any math so that enough bytes are in
 //     flight per SM to cover HBM latency (needs ~35 KB/SM in flight at 6.5 TB/s);
 //   * all intermediates of a point live in registers; outputs are stored as soon as a vector is done;
 //   * tiles are handed to CTAs round-robin (grid-stride), grid sized as SMs x CTAs-per-SM;
@@ -17,43 +17,6 @@
 #include <cuda_runtime.h>
 
 #include "ek_thermo_math.cuh"
-
-#ifndef EK_UNROLL
-#define EK_UNROLL 2  // 16-byte vectors per input per thread per tile
-#endif
-#ifndef EK_PIPELINE
-#define EK_PIPELINE 0  // 1: prefetch the next tile into a second register set before computing the current one.
-                       // Measured on B200 (profiles/r01_kbench_pipeline_unroll_variants.log): no gain over 0 -- 32 resident
-                       // warps/SM with 2 front-loaded vectors per input already cover the HBM latency -- so it stays off.
-#endif
-#ifndef EK_MAX_THREADS
-#define EK_MAX_THREADS 256
-#endif
-#ifndef EK_DEFER_TILE
-#define EK_DEFER_TILE 0
-#endif
-#ifndef EK_PF_DIST
-#define EK_PF_DIST 2  // tiles ahead of the current one that prefetch_tile_l2 asks L2 for (functors with PREFETCH_NEXT)
-#endif
-#ifndef EK_HEAVY_MIN_CTAS
-#define EK_HEAVY_MIN_CTAS 3  // resident CTAs per SM for the functors that declare HEAVY (the fused suites, ept / ept + wet bulb):
-                             // 80 registers instead of 64 -- no spills in their ~200-instruction bodies -- and, with the L2 prefetch
-                             // two tiles ahead covering what the fourth CTA's loads covered, 3-6 % more of the roofline
-                             // (profiles/r02_ab_ew.log: suite 0.886 -> 0.923, ept + wet bulb 0.80 -> 0.86, single pass 0.76 -> 0.84);
-                             // the short single-output kernels lose 7-10 % with it (theta 0.974 -> 0.871) and keep EK_MIN_CTAS
-#endif
-#ifndef EK_LAST_SCALAR_LOOP
-#define EK_LAST_SCALAR_LOOP 1  // a tile loop specialised for "every input an array, the last one a scalar" (pressure-level data)
-#endif
-#ifndef EK_PDL
-#define EK_PDL 1  // programmatic dependent launch: a streaming kernel lets its successor in the stream start (launch latency, CTA
-                  // scheduling, the copy of the lean tables) while its own last CTAs drain; the successor waits for the
-                  // predecessor's completion and memory flush before it touches a field (griddepcontrol.wait).  One launch per
-                  // 1 M-point level, theta + rh: eager 13.3 -> 11.3 us, graph replay 11.8 -> 11.0 us (profiles/r02f_kbench_levels.log)
-#endif
-#ifndef EK_MIN_CTAS
-#define EK_MIN_CTAS 4  // <= 64 registers per thread: 4 CTAs = 32 warps per SM hide the fp64 dependency chains
-#endif
 
 namespace ek {
 
@@ -100,7 +63,16 @@ constexpr unsigned kSmemBytes = 2 * 8 * EK_LOG_TAB_N + 8 * EK_EXP_TAB_N;  // lea
 constexpr unsigned kSmemBytes = 0;
 #endif
 
-constexpr int kThreads = EK_MAX_THREADS;  // CTA size is a compile-time constant: tile offsets become immediates
+constexpr int kThreads = 256;  // CTA size is a compile-time constant: tile offsets become immediates
+constexpr int kUnroll = 2;     // 16-byte vectors per input per thread per tile (1 vector: suite +1 %, theta -13 %)
+constexpr int kPfDist = 2;     // tiles ahead of the current one that prefetch_tile_l2 asks L2 for (functors with PREFETCH_NEXT);
+                               // 1 or 3 tiles ahead: suite 0.92 -> 0.89
+constexpr int kMinCtas = 4;    // <= 64 registers per thread: 4 CTAs = 32 warps per SM hide the fp64 dependency chains
+// Resident CTAs per SM for the functors that declare HEAVY (the fused suites, ept / ept + wet bulb): 80 registers instead of 64 --
+// no spills in their ~200-instruction bodies -- and, with the L2 prefetch two tiles ahead covering what the fourth CTA's loads
+// covered, 3-6 % more of the roofline (profiles/r02_ab_ew.log: suite 0.886 -> 0.923, ept + wet bulb 0.80 -> 0.86, single pass
+// 0.76 -> 0.84); the short single-output kernels lose 7-10 % with it (theta 0.974 -> 0.871) and keep kMinCtas.
+constexpr int kHeavyMinCtas = 3;
 
 template <typename T> __device__ __forceinline__ bool is_nan_val(T v) { return v != v; }
 
@@ -205,21 +177,21 @@ __device__ __forceinline__ void points_n(const T (&a)[N][Op::NIN], T (&r)[N][Op:
 #endif
 }
 
-// 16-byte vectors per input per thread per tile: EK_UNROLL unless the functor declares `UNROLL` (the one-step Newton solve keeps
+// 16-byte vectors per input per thread per tile: kUnroll unless the functor declares `UNROLL` (the one-step Newton solve keeps
 // one vector in flight: its ~550-instruction body needs the registers, and without spills it runs 8-12 % faster).
 template <class Op, class = void> struct UnrollOf {
-    static constexpr int value = EK_UNROLL;
+    static constexpr int value = kUnroll;
 };
 template <class Op> struct UnrollOf<Op, decltype((void)Op::UNROLL)> {
-    static constexpr int value = Op::UNROLL > 0 ? Op::UNROLL : EK_UNROLL;
+    static constexpr int value = Op::UNROLL > 0 ? Op::UNROLL : kUnroll;
 };
 
 // The "last input is a scalar" tile loop (load_tile ALLARR == 2) unless the functor opts out with LAST_SCALAR_LOOP = false
 template <class Op, class = void> struct LastScalarLoopOf {
-    static constexpr bool value = EK_LAST_SCALAR_LOOP != 0;
+    static constexpr bool value = true;
 };
 template <class Op> struct LastScalarLoopOf<Op, decltype((void)Op::LAST_SCALAR_LOOP)> {
-    static constexpr bool value = EK_LAST_SCALAR_LOOP != 0 && Op::LAST_SCALAR_LOOP;
+    static constexpr bool value = Op::LAST_SCALAR_LOOP;
 };
 
 template <class Op, class = void> struct DeferColdOf {
@@ -229,12 +201,12 @@ template <class Op> struct DeferColdOf<Op, decltype((void)Op::DEFER_COLD)> {
     static constexpr bool value = Op::DEFER_COLD;
 };
 
-// Resident CTAs per SM a functor's register budget is sized for: EK_MIN_CTAS, or EK_HEAVY_MIN_CTAS where the functor says HEAVY.
+// Resident CTAs per SM a functor's register budget is sized for: kMinCtas, or kHeavyMinCtas where the functor says HEAVY.
 template <class Op, class = void> struct MinCtasOf {
-    static constexpr int value = EK_MIN_CTAS;
+    static constexpr int value = kMinCtas;
 };
 template <class Op> struct MinCtasOf<Op, decltype((void)Op::HEAVY)> {
-    static constexpr int value = Op::HEAVY ? (Op::HEAVY > 1 ? Op::HEAVY : EK_HEAVY_MIN_CTAS) : EK_MIN_CTAS;  // HEAVY > 1: that many CTAs
+    static constexpr int value = Op::HEAVY ? kHeavyMinCtas : kMinCtas;
 };
 
 // The inputs of one tile, per thread: UNROLL 16-byte vectors of every input array, in registers.
@@ -303,56 +275,6 @@ __device__ __forceinline__ void compute_store_tile(const TileRegs<Op, T, UNROLL>
     constexpr int NOUT = Op::NOUT;
     constexpr int VEC = Vec16<T>::N;
     constexpr int VSTRIDE = kThreads * VEC;
-#if EK_DEFER_TILE
-    if constexpr (DeferColdOf<Op>::value && EK_LEAN_DEVICE && !IsBatch<Op>::value) {
-        // experiment: ALL points of the tile (UNROLL x VEC) through the fast functor back to back, NaN checks afterwards
-        T res[UNROLL][VEC][NOUT];
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u)
-#pragma unroll
-            for (int v = 0; v < VEC; ++v) {
-                T a[NIN];
-#pragma unroll
-                for (int k = 0; k < NIN; ++k) a[k] = r.x[k][u][v];
-#pragma unroll
-                for (int o = 0; o < NOUT; ++o) res[u][v][o] = T(0);
-                Op::template apply<T>(a, res[u][v], P);
-            }
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-            T y[NOUT][VEC];
-#pragma unroll
-            for (int v = 0; v < VEC; ++v) {
-                if ((sizeof(T) == 8 || ColdF32<Op>::value) && __builtin_expect(any_nan<NOUT>(res[u][v]), 0)) {
-                    T a2[NIN], r2[NOUT];
-#pragma unroll
-                    for (int k = 0; k < NIN; ++k) a2[k] = r.x[k][u][v];
-#pragma unroll
-                    for (int o = 0; o < NOUT; ++o) r2[o] = res[u][v][o];
-                    cold_point<OpE, T>(a2, r2, P, array_mask);
-#pragma unroll
-                    for (int o = 0; o < NOUT; ++o) res[u][v][o] = r2[o];
-                }
-#pragma unroll
-                for (int o = 0; o < NOUT; ++o) y[o][v] = res[u][v][o];
-            }
-#pragma unroll
-            for (int o = 0; o < NOUT; ++o) {
-                const bool w = Op::STATIC_MASK ? (((Op::STATIC_MASK >> o) & 1u) != 0) : (out.p[o] != nullptr);
-                if (w) {
-                    T* dst = static_cast<T*>(out.p[o]) + base + u * VSTRIDE;
-                    if (VECOK) {
-                        Vec16<T>::store(dst, y[o]);
-                    } else {
-#pragma unroll
-                        for (int v = 0; v < VEC; ++v) __stcs(dst + v, y[o][v]);
-                    }
-                }
-            }
-        }
-        return;
-    }
-#endif
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
         T y[NOUT][VEC];
@@ -424,9 +346,9 @@ __device__ __forceinline__ void compute_store_tile(const TileRegs<Op, T, UNROLL>
     }
 }
 
-// Tiles are handed to CTAs round-robin.  The loop is software-pipelined in registers: the loads of a CTA's NEXT
-// tile are issued before the math of the current one, so every warp keeps HBM requests in flight while it
-// computes (two register sets, A and B, alternate; no dynamic register indexing).
+// Tiles are handed to CTAs round-robin; a tile's loads are all issued before its math.  Loading the NEXT tile into a second
+// register set before computing the current one measured no gain on B200 (profiles/r01_kbench_pipeline_unroll_variants.log):
+// 32 resident warps/SM with 2 front-loaded vectors per input already cover the HBM latency.
 template <class Op, class OpE, typename T, int UNROLL, bool VECOK, int ALLARR>
 __device__ __forceinline__ void tile_loop(const InArgs<Op::NIN>& in, const OutArgs<Op::NOUT>& out, const int64_t ntiles, const Params& P,
                                           const uint32_t array_mask) {
@@ -435,45 +357,23 @@ __device__ __forceinline__ void tile_loop(const InArgs<Op::NIN>& in, const OutAr
     const int64_t toff = (int64_t)threadIdx.x * Vec16<T>::N;
     int64_t ta = blockIdx.x;
     if (ta >= ntiles) return;
-#if EK_PIPELINE
-    TileRegs<Op, T, UNROLL> A, B;
-    load_tile<Op, T, UNROLL, VECOK, ALLARR>(A, in, ta * TILE + toff);
-    for (;;) {
-        const int64_t tb = ta + G;
-        const bool hb = tb < ntiles;
-        if (hb) load_tile<Op, T, UNROLL, VECOK, ALLARR>(B, in, tb * TILE + toff);
-        compute_store_tile<Op, OpE, T, UNROLL, VECOK>(A, out, ta * TILE + toff, P, array_mask);
-        if (!hb) break;
-        ta = tb + G;
-        const bool ha = ta < ntiles;
-        if (ha) load_tile<Op, T, UNROLL, VECOK, ALLARR>(A, in, ta * TILE + toff);
-        compute_store_tile<Op, OpE, T, UNROLL, VECOK>(B, out, tb * TILE + toff, P, array_mask);
-        if (!ha) break;
-    }
-#else
     for (; ta < ntiles; ta += G) {
         TileRegs<Op, T, UNROLL> A;
         load_tile<Op, T, UNROLL, VECOK, ALLARR>(A, in, ta * TILE + toff);
-        if (Op::PREFETCH_NEXT && ta + EK_PF_DIST * G < ntiles) prefetch_tile_l2<Op, T, UNROLL>(in, (ta + EK_PF_DIST * G) * TILE + toff);
+        if (Op::PREFETCH_NEXT && ta + kPfDist * G < ntiles) prefetch_tile_l2<Op, T, UNROLL>(in, (ta + kPfDist * G) * TILE + toff);
         compute_store_tile<Op, OpE, T, UNROLL, VECOK>(A, out, ta * TILE + toff, P, array_mask);
     }
-#endif
 }
 
-// Programmatic dependent launch (sm_90+).  pdl_release: the next kernel of the stream may be scheduled as soon as every CTA of
-// this grid has started; pdl_acquire: wait until the previous kernel of the stream has completed and its writes are visible.
-// Everything that reads or writes a field comes after pdl_acquire; only the table copy (immutable data) runs before it.
-// Both are no-ops for a kernel launched without the programmatic-serialization attribute.
-__device__ __forceinline__ void pdl_release() {
-#if EK_PDL
-    asm volatile("griddepcontrol.launch_dependents;");
-#endif
-}
-__device__ __forceinline__ void pdl_acquire() {
-#if EK_PDL
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
-}
+// Programmatic dependent launch (sm_90+): a streaming kernel lets its successor in the stream start (launch latency, CTA
+// scheduling, the copy of the lean tables) while its own last CTAs drain.  One launch per 1 M-point level, theta + rh: eager
+// 13.3 -> 11.3 us, graph replay 11.8 -> 11.0 us (profiles/r02f_kbench_levels.log).
+// pdl_release: the next kernel of the stream may be scheduled as soon as every CTA of this grid has started; pdl_acquire: wait
+// until the previous kernel of the stream has completed and its writes are visible.  Everything that reads or writes a field
+// comes after pdl_acquire; only the table copy (immutable data) runs before it.  Both are no-ops for a kernel launched without
+// the programmatic-serialization attribute.
+__device__ __forceinline__ void pdl_release() { asm volatile("griddepcontrol.launch_dependents;"); }
+__device__ __forceinline__ void pdl_acquire() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 template <class Op, class OpE, typename T, int UNROLL>
 __global__ void __launch_bounds__(kThreads, MinCtasOf<Op>::value)
@@ -559,8 +459,8 @@ __global__ void __launch_bounds__(kThreads, MinCtasOf<Op>::value)
 #pragma unroll
         for (int o = 0; o < NOUT; ++o) out.p[o] = ((B.out_mask >> o) & 1u) ? B.out[o][seg] : nullptr;
         auto prefetch_next = [&]() {
-            if (Op::PREFETCH_NEXT) {  // the CTA's tile EK_PF_DIST rounds ahead, possibly in a later segment
-                const int64_t nt = tile + EK_PF_DIST * (int64_t)gridDim.x;
+            if (Op::PREFETCH_NEXT) {  // the CTA's tile kPfDist rounds ahead, possibly in a later segment
+                const int64_t nt = tile + kPfDist * (int64_t)gridDim.x;
                 if (nt < ntiles) {
                     const int nseg = (int)(nt / tiles_per_seg);
                     InArgs<NIN> nin;

@@ -8,12 +8,16 @@
 // need (correct rounding of the quotient, denormal results):
 //
 //   rcp_/div_  MUFU.RCP64H seed (2^-19.9, measured: tools/probe_mufu.cu) + one cubic Newton step: <= 2 ulp
-//   log_       2^L-entry {1/c, ln c} table, r = z/c - 1 (|r| < 2^-(L+1)), log1p polynomial of degree 4 (L >= 10),
-//              5 (L >= 8) or 6: ~1 ulp (abs 2e-16)
-//   exp_       2^E-entry 2^(j/2^E) table, polynomial of degree 3 (E >= 11), 4 (E >= 8) or 5 on |r| <= ln2/2^(E+1): ~1 ulp
-//   (L = EK_LOG_TAB_BITS, E = EK_EXP_TAB_BITS, set by tools/gen_lean_tables.py; the shipped tables are L = 10, E = 11:
-//   32 KB of shared memory per CTA buy two FP64 instructions per log_ and per exp_)
+//   log_       2^10-entry {1/c, ln c} table, r = z/c - 1 (|r| < 2^-11), log1p polynomial of degree 4, k*ln2 added as a
+//              hi/lo pair: ~1 ulp (abs 2e-16)
+//   exp_       2^11-entry 2^(j/2^11) table, polynomial of degree 3 on |r| <= ln2/2^12: ~1 ulp
+//   (the tables come from tools/gen_lean_tables.py: their 32 KB of shared memory per CTA buy two FP64 instructions per log_
+//   and per exp_)
 //   pow_       exp_(y * log_(x)): relative error ~ |y ln x| * 2e-16
+//
+// The constants whose low 32 bits are zero (+-0.5, -0.25, the 1.5*2^52 rounding constant) are written as literals: they
+// become 32-bit immediates of DFMA / DADD instead of occupying uniform registers, and a polynomial step fma(r, c1, c0) no
+// longer needs two constant operands (only one fits an instruction).
 //
 // The fp64 primitives are branch-free.  Outside their fast domain (x <= 0, denormal, inf, NaN for log_; |x| >= 708
 // or NaN for exp_; b = 0, denormal, inf, NaN for rcp_) they answer NaN; the kernel recomputes any point whose
@@ -26,31 +30,9 @@
 #pragma once
 #include "ek_thermo_lean_tables.inc"
 
-#if EK_LOG_TAB_BITS >= 10
-#define EK_LOG_DEG 4
-#elif EK_LOG_TAB_BITS >= 8
-#define EK_LOG_DEG 5
-#else
-#define EK_LOG_DEG 6
-#endif
-#if EK_EXP_TAB_BITS >= 11
-#define EK_EXP_DEG 3
-#elif EK_EXP_TAB_BITS >= 8
-#define EK_EXP_DEG 4
-#else
-#define EK_EXP_DEG 5
-#endif
-#ifndef EK_LEAN_LOG_HILO
-#define EK_LEAN_LOG_HILO 1  // 1: k*ln2 added as a hi/lo pair (abs error of log_ ~2e-16); 0: one FMA less, ~1.5 ulp of the result
-#endif
-#ifndef EK_LEAN_REGROUP
-#define EK_LEAN_REGROUP 1  // 1: three regroupings that save one FP64 operation each (t_from_es, the Exner exponent, the "direct" fit)
-#endif
-#ifndef EK_LEAN_IMM
-#define EK_LEAN_IMM 1  // 1: the constants whose low 32 bits are zero (+-0.5, -0.25, the 1.5*2^52 rounding constant) are written as
-                       // literals: they become 32-bit immediates of DFMA / DADD instead of occupying uniform registers, and a
-                       // polynomial step fma(r, c1, c0) no longer needs two constant operands (only one fits an instruction)
-#endif
+// the polynomial degrees of log_ and exp_ are chosen for these table sizes
+static_assert(EK_LOG_TAB_BITS == 10 && EK_LOG_TAB_N == 1024 && EK_EXP_TAB_BITS == 11 && EK_EXP_TAB_N == 2048,
+              "log_ / exp_ need 2^10-entry log and 2^11-entry exp tables");
 
 namespace ek {
 namespace lean {
@@ -131,54 +113,27 @@ __device__ __forceinline__ double log_(double x) {
     const double r = fma(z, tc.x, -1.0);
     const double kd = (double)k;
     const double r2 = r * r;
-    // log1p(r) = r + r^2 s(r), s = -1/2 + r/3 - r^2/4 + ... (Estrin: short dependency chains)
-#if EK_LOG_DEG == 6
-    double p = fma(r, kLog[4], kLog[3]);
-    const double q = fma(r, kLog[2], kLog[1]);
-    p = fma(r2, p, q);
-    const double s = fma(r, p, kLog[0]);
-#elif EK_LOG_DEG == 5
-    const double s = fma(r2, fma(r, kLog[3], kLog[2]), fma(r, kLog[1], kLog[0]));
-#elif EK_LEAN_IMM
+    // log1p(r) = r + r^2 s(r), s = -1/2 + r/3 - r^2/4 (Estrin: short dependency chains)
     const double s = fma(r2, -0.25, fma(r, kLog[1], -0.5));
-#else
-    const double s = fma(r2, kLog[2], fma(r, kLog[1], kLog[0]));
-#endif
-#if EK_LEAN_LOG_HILO
+    // k*ln2 as a hi/lo pair (abs error ~2e-16); one FMA with ln2 is ~1.5 ulp of the result and measured within noise on B200
+    // (ept + wet bulb +3 %, suites -1.5 %)
     const double t1 = fma(kd, kRed[3], tc.y);
     const double t2 = fma(kd, kRed[4], r);
     const double y = fma(r2, s, t2) + t1;
-#else
-    const double y = fma(r2, s, r) + fma(kd, kRed[8], tc.y);
-#endif
     return __hiloint2double(bad ? 0x7ff80000 : __double2hiint(y), __double2loint(y));
 }
 
 __device__ __forceinline__ double exp_(double x) {
     const bool bad = (unsigned)(__double2hiint(x) & 0x7fffffff) >= 0x40862000u;  // |x| >= 708, inf, NaN: answer NaN
-#if EK_LEAN_IMM
     const double t = fma(x, kRed[0], 0x1.8p52);
     const int ki = __double2loint(t);
     const double kd = t - 0x1.8p52;
-#else
-    const double t = fma(x, kRed[0], kRed[5]);
-    const int ki = __double2loint(t);
-    const double kd = t - kRed[5];
-#endif
     double r = fma(kd, -kRed[1], x);
     r = fma(kd, -kRed[2], r);
     const double T = lds_exp(ki & (EK_EXP_TAB_N - 1));
     const double r2 = r * r;
-    // e^r - 1 = r + r^2 s(r), s = 1/2 + r/6 + r^2/24 + r^3/120
-#if EK_EXP_DEG == 5
-    const double s = fma(r2, fma(r, kExp[3], kExp[2]), fma(r, kExp[1], kExp[0]));
-#elif EK_EXP_DEG == 4
-    const double s = fma(r2, kExp[2], fma(r, kExp[1], kExp[0]));
-#elif EK_LEAN_IMM
+    // e^r - 1 = r + r^2 s(r), s = 1/2 + r/6
     const double s = fma(r, kExp[1], 0.5);
-#else
-    const double s = fma(r, kExp[1], kExp[0]);
-#endif
     const double p = fma(r2, s, r);
     const double y = fma(T, p, T);
     return __hiloint2double(bad ? 0x7ff80000 : __double2hiint(y) + ((ki >> EK_EXP_TAB_BITS) << 20), __double2loint(y));
@@ -195,11 +150,7 @@ __device__ __forceinline__ double log_p0_over(double x);
 __device__ __forceinline__ float log_p0_over(float x) { return (float)EK_LOG_P0 - __logf(x); }
 
 // kappa * ln(p0 / x): the exponent of the Exner factor, for callers that fold it into a larger exponential
-#if EK_LEAN_REGROUP
 __device__ __forceinline__ double kappa_log_p0_over(double x) { return fma(-::ek::kCdev.kappa, log_(x), kRed[9]); }  // kRed[9] = kappa ln p0
-#else
-__device__ __forceinline__ double kappa_log_p0_over(double x) { return ::ek::kCdev.kappa * (kRed[6] - log_(x)); }
-#endif
 __device__ __forceinline__ float kappa_log_p0_over(float x) { return (float)::ek::kC.kappa * ((float)EK_LOG_P0 - __logf(x)); }
 
 __device__ __forceinline__ double log_p0_over(double x) { return kRed[6] - log_(x); }

@@ -34,9 +34,6 @@
 #ifndef EK_LEAN_MATH
 #define EK_LEAN_MATH 0
 #endif
-#ifndef EK_LEAN_DJ_MERGED
-#define EK_LEAN_DJ_MERGED 1  // lean build: Davies-Jones lcl fit with its constants merged (see lcl_t_davies)
-#endif
 
 #if EK_LEAN_MATH && defined(__CUDA_ARCH__)
 #define EK_LEAN_DEVICE 1

@@ -5,7 +5,7 @@
 
 The tile loop is taken as the span between the first LDG.E.EF.128 and the last backward branch after the last STG.E.EF.128
 of the kernel; blocks that end in a CALL (the out-of-line exact recompute) are left out.  Counts are per loop iteration
-(= EK_UNROLL x VEC points); straight-line code only -- kernels with uniform branches inside the loop over-count.
+(= kUnroll x VEC points); straight-line code only -- kernels with uniform branches inside the loop over-count.
 """
 import collections
 import re
