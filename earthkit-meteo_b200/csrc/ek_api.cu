@@ -72,6 +72,10 @@ template <typename T> int ek_suite_launch_ttdp(const ek_operand* ins, void* cons
 template <typename T>
 int ek_suite_launch_hybrid(const void* t, const void* q, const void* sp, const void* A, const void* B, int nlev, int64_t npl, void* const* outs,
                            uint32_t out_mask, int ept_method, void* stream);
+template <typename T>
+int ek_suite_launch_hybrid_geo(const void* t, const void* q, const void* sp, const void* zs, const void* A, const void* B, int nlev, int64_t npl,
+                               void* const* outs, uint32_t out_mask, int ept_method, int top_toa, double alpha_top, void* const* cols,
+                               int height_mode, void* stream);
 
 // ---- host-buffer pipeline ---------------------------------------------------------------------------
 namespace {
@@ -102,8 +106,8 @@ struct StreamSet {
     }
 };
 
-int count_outputs(const char* what, void* const* h_outs, uint32_t out_mask, int* n_out) {
-    if (out_mask == 0 || out_mask >= (1u << S_NSLOTS)) return set_error(EK_ERR_ARG, "%s: out_mask=0x%x", what, out_mask);
+int count_outputs(const char* what, void* const* h_outs, uint32_t out_mask, int* n_out, bool allow_none = false) {
+    if ((out_mask == 0 && !allow_none) || out_mask >= (1u << S_NSLOTS)) return set_error(EK_ERR_ARG, "%s: out_mask=0x%x", what, out_mask);
     *n_out = 0;
     for (int k = 0; k < S_NSLOTS; ++k)
         if ((out_mask >> k) & 1u) {
@@ -169,21 +173,30 @@ EK_API(host_suite,
 // The hybrid-level suite fed from HOST arrays: t, q and every output are [nlev, npl] host arrays, sp is [npl], A / B the
 // nlev + 1 half-level coefficients.  The pressure field never exists on either side of PCIe: 16 + 8/nlev bytes per point
 // travel to the device instead of 24.  Chunks are column ranges of all levels; each array of a chunk moves as one 2-D
-// copy (nlev rows of chunk-columns, host pitch npl).
+// copy (nlev rows of chunk-columns, host pitch npl).  With column outputs (h_cols: thickness, z, height; NULL or any entry
+// NULL for none) the chunks run the suite + geopotential kernel instead, and zs travels as one more [npl] row when an output
+// needs it.
 template <typename T>
-static int impl_host_suite_tq_hybrid(const void* h_t, const void* h_q, const void* h_sp, const void* h_A, const void* h_B, int nlev, int64_t npl,
-                                     void* const* h_outs, uint32_t out_mask, int ept_method, void* workspace, size_t workspace_bytes,
-                                     int n_slots) {
-    const char* what = "host_suite_tq_hybrid";
+static int host_suite_tq_hybrid(const char* what, const void* h_t, const void* h_q, const void* h_sp, const void* h_zs, const void* h_A,
+                                const void* h_B, int nlev, int64_t npl, void* const* h_outs, uint32_t out_mask, int ept_method, int top_toa,
+                                double alpha_top, void* const* h_cols, int height_mode, void* workspace, size_t workspace_bytes, int n_slots) {
     if (!h_t || !h_q || !h_sp || !h_A || !h_B || !h_outs || !workspace) return set_error(EK_ERR_ARG, "%s: NULL buffer", what);
     if (nlev < 1 || npl < 0 || n_slots < 1 || n_slots > 16) return set_error(EK_ERR_ARG, "%s: nlev=%d npl=%lld n_slots=%d", what, nlev, (long long)npl, n_slots);
+    int n_col = 0;
+    for (int k = 0; k < 3; ++k) n_col += (h_cols && h_cols[k]) ? 1 : 0;
+    const bool geo = n_col > 0;
+    if (geo && h_cols[2] && (height_mode < EK_HM_THICKNESS || height_mode > EK_HM_GEOM_GROUND))
+        return set_error(EK_ERR_ENUM, "%s: invalid height mode %d", what, height_mode);
+    const bool zs_row = geo && (h_cols[1] || (h_cols[2] && height_mode != EK_HM_THICKNESS && height_mode != EK_HM_GH_GROUND));
+    if (zs_row && !h_zs) return set_error(EK_ERR_ARG, "%s: this output needs the surface geopotential zs", what);
     int n_out = 0;
-    if (int rc = count_outputs(what, h_outs, out_mask, &n_out)) return rc;
+    if (int rc = count_outputs(what, h_outs, out_mask, &n_out, geo)) return rc;
     if (npl == 0) return EK_OK;
     if (!aligned16(workspace)) return set_error(EK_ERR_ARG, "%s: workspace must be 16-byte aligned", what);
     const size_t coef = (((size_t)(nlev + 1) * sizeof(T) + 255u) / 256u) * 256u;  // A, then B, at the start of the workspace
     if (workspace_bytes <= 2 * coef) return set_error(EK_ERR_PIPE, "%s: workspace of %zu bytes is too small", what, workspace_bytes);
-    const int64_t rows = (int64_t)(2 + n_out) * nlev + 1;  // device rows of one chunk: t, q, outputs (nlev each) + sp
+    // device rows of one chunk: t, q, outputs, column outputs (nlev each) + sp (+ zs)
+    const int64_t rows = (int64_t)(2 + n_out + n_col) * nlev + 1 + (zs_row ? 1 : 0);
     int64_t chunk = (int64_t)((workspace_bytes - 2 * coef) / ((size_t)n_slots * rows * sizeof(T)));
     chunk -= chunk % 1024;  // whole vectors, 16-byte aligned rows
     if (chunk <= 0) return set_error(EK_ERR_PIPE, "%s: workspace of %zu bytes is too small for %d slots of %d levels", what, workspace_bytes, n_slots, nlev);
@@ -224,22 +237,57 @@ static int impl_host_suite_tq_hybrid(const void* h_t, const void* h_q, const voi
         e = cudaMemcpy2DAsync(d_t, dpitch, static_cast<const T*>(h_t) + done, hpitch, dpitch, (size_t)nlev, cudaMemcpyHostToDevice, st);
         if (e == cudaSuccess) e = cudaMemcpy2DAsync(d_q, dpitch, static_cast<const T*>(h_q) + done, hpitch, dpitch, (size_t)nlev, cudaMemcpyHostToDevice, st);
         if (e == cudaSuccess) e = cudaMemcpyAsync(d_sp, static_cast<const T*>(h_sp) + done, dpitch, cudaMemcpyHostToDevice, st);
+        T* d_zs = zs_row ? d_sp + chunk : nullptr;
+        if (e == cudaSuccess && zs_row) e = cudaMemcpyAsync(d_zs, static_cast<const T*>(h_zs) + done, dpitch, cudaMemcpyHostToDevice, st);
         if (e != cudaSuccess) return set_error((int)e, "%s: H2D copy: %s", what, cudaGetErrorString(e));
         void* douts[S_NSLOTS];
         int j = 0;
-        T* d_out0 = d_sp + chunk;
+        T* d_out0 = d_sp + (zs_row ? 2 : 1) * chunk;
         for (int k = 0; k < S_NSLOTS; ++k) douts[k] = ((out_mask >> k) & 1u) ? (void*)(d_out0 + (int64_t)(j++) * nlev * chunk) : nullptr;
-        int rc = ek_suite_launch_hybrid<T>(d_t, d_q, d_sp, dA, dB, nlev, m, douts, out_mask, ept_method, st);
+        void* dcols[3];
+        for (int k = 0; k < 3; ++k) dcols[k] = (geo && h_cols[k]) ? (void*)(d_out0 + (int64_t)(j++) * nlev * chunk) : nullptr;
+        int rc = geo ? ek_suite_launch_hybrid_geo<T>(d_t, d_q, d_sp, d_zs, dA, dB, nlev, m, douts, out_mask, ept_method, top_toa, alpha_top, dcols,
+                                                     height_mode, st)
+                     : ek_suite_launch_hybrid<T>(d_t, d_q, d_sp, dA, dB, nlev, m, douts, out_mask, ept_method, st);
         if (rc != EK_OK) return rc;
-        for (int k = 0; k < S_NSLOTS; ++k)
-            if (douts[k]) {
-                e = cudaMemcpy2DAsync(static_cast<T*>(h_outs[k]) + done, hpitch, douts[k], dpitch, dpitch, (size_t)nlev, cudaMemcpyDeviceToHost, st);
+        for (int k = 0; k < S_NSLOTS + 3; ++k) {
+            void* h = k < S_NSLOTS ? h_outs[k] : (geo ? h_cols[k - S_NSLOTS] : nullptr);
+            void* d = k < S_NSLOTS ? douts[k] : dcols[k - S_NSLOTS];
+            if (d) {
+                e = cudaMemcpy2DAsync(static_cast<T*>(h) + done, hpitch, d, dpitch, dpitch, (size_t)nlev, cudaMemcpyDeviceToHost, st);
                 if (e != cudaSuccess) return set_error((int)e, "%s: D2H copy: %s", what, cudaGetErrorString(e));
             }
+        }
     }
     return ss.drain();
+}
+
+template <typename T>
+static int impl_host_suite_tq_hybrid(const void* h_t, const void* h_q, const void* h_sp, const void* h_A, const void* h_B, int nlev, int64_t npl,
+                                     void* const* h_outs, uint32_t out_mask, int ept_method, void* workspace, size_t workspace_bytes,
+                                     int n_slots) {
+    return host_suite_tq_hybrid<T>("host_suite_tq_hybrid", h_t, h_q, h_sp, nullptr, h_A, h_B, nlev, npl, h_outs, out_mask, ept_method, 0, 0.0,
+                                   nullptr, 0, workspace, workspace_bytes, n_slots);
 }
 EK_API(host_suite_tq_hybrid,
        (const void* h_t, const void* h_q, const void* h_sp, const void* h_A, const void* h_B, int nlev, int64_t npl, void* const* h_outs,
         uint32_t out_mask, int ept_method, void* workspace, size_t workspace_bytes, int n_slots),
        (h_t, h_q, h_sp, h_A, h_B, nlev, npl, h_outs, out_mask, ept_method, workspace, workspace_bytes, n_slots))
+
+template <typename T>
+static int impl_host_suite_tq_hybrid_geo(const void* h_t, const void* h_q, const void* h_sp, const void* h_zs, const void* h_A, const void* h_B,
+                                         int nlev, int64_t npl, void* const* h_outs, uint32_t out_mask, int ept_method, int top_toa,
+                                         double alpha_top, void* h_thickness, void* h_z, void* h_height, int height_mode, void* workspace,
+                                         size_t workspace_bytes, int n_slots) {
+    const char* what = "host_suite_tq_hybrid_geo";
+    if (!h_thickness && !h_z && !h_height) return set_error(EK_ERR_ARG, "%s: no column output given (use host_suite_tq_hybrid)", what);
+    void* const cols[3] = {h_thickness, h_z, h_height};
+    return host_suite_tq_hybrid<T>(what, h_t, h_q, h_sp, h_zs, h_A, h_B, nlev, npl, h_outs, out_mask, ept_method, top_toa, alpha_top, cols,
+                                   height_mode, workspace, workspace_bytes, n_slots);
+}
+EK_API(host_suite_tq_hybrid_geo,
+       (const void* h_t, const void* h_q, const void* h_sp, const void* h_zs, const void* h_A, const void* h_B, int nlev, int64_t npl,
+        void* const* h_outs, uint32_t out_mask, int ept_method, int top_toa, double alpha_top, void* h_thickness, void* h_z, void* h_height,
+        int height_mode, void* workspace, size_t workspace_bytes, int n_slots),
+       (h_t, h_q, h_sp, h_zs, h_A, h_B, nlev, npl, h_outs, out_mask, ept_method, top_toa, alpha_top, h_thickness, h_z, h_height, height_mode,
+        workspace, workspace_bytes, n_slots))

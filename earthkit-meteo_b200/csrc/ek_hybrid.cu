@@ -39,6 +39,14 @@ constexpr int kColLevels = 2;       // column kernel, computed alpha/delta: leve
 constexpr int kColMinCtas = 3;      // column kernel: resident CTAs per SM
 constexpr int kColMinCtasGeom = 4;  // column kernel, geometric-height forms: resident CTAs per SM
 constexpr int kColPfDist = 2;       // column kernel: groups of levels the L2 prefetch runs ahead
+// suite + geopotential walk, measured on B200 at 1000 W, O1280 x 137 fp64, 5 outputs + z, fused time / the two launches it replaces
+// in the same process (profiles/r03_kbench_geo_sweep_f64.log): 2 levels in flight 0.95 (other runs 0.92-0.94), 1 level 0.92, 3 levels
+// 1.01; 3 CTAs per SM (80 registers) 1.09; prefetch 1 or 3 groups ahead 0.93 / 0.95.  1 and 2 levels and the prefetch distances are
+// inside the run-to-run spread; 2 levels at 2 CTAs (128 registers) and 2 groups ahead, the column kernel's values, are kept.  With
+// them (profiles/r03_kbench_geo_f64.log, r03_kbench_geo_f32.log): fp64 11.60 ms = 0.75 of the 64 B/pt roofline, fp32 4.96 ms = 0.88.
+constexpr int kGeoLevels = 2;       // suite + geopotential walk: levels whose t/q loads are in flight per thread
+constexpr int kGeoMinCtas = 2;      // suite + geopotential walk: resident CTAs per SM
+constexpr int kGeoPfDist = 2;       // suite + geopotential walk: groups of levels the L2 prefetch runs ahead
 
 namespace {
 
@@ -402,6 +410,120 @@ __global__ void __launch_bounds__(kThreads, (MODE >= EK_HM_GEOM_SEA ? kColMinCta
     }
 }
 
+struct SuiteGeoArgs {
+    const void *t, *q, *sp, *zs, *A, *B;  // t, q: [nlev, npl]; sp, zs: [npl] (zs may be NULL when no output adds it); A, B: nlev + 1
+    void* outs[S_NSLOTS];
+    void* p_out;                          // optional: the full-level pressure
+    void *thickness, *z, *height;         // optional column outputs [nlev, npl]
+    int nlev;
+    int64_t npl;
+    int top_toa;   // field-wide any(p_half[0] <= 0.1) (V:678)
+    double alpha_top;
+    int mode;      // HeightMode of `height`
+};
+
+// The (t, q, p) suite and the geopotential of the same levels in one walk: one thread per VEC columns from the bottom level to the
+// top one, as column_geopotential_kernel (computed alpha/delta).  A level forms its top half-level pressure once; the full-level
+// pressure (the same two operands as suite_hybrid_kernel: bit-identical to pressure_on_hybrid_levels), delta and alpha all come
+// from it and the half level below.  The three column outputs are forms of the same dphi; the height form is a warp-uniform
+// run-time value (column_geopotential_kernel's MODE = -1 expression).
+template <class Op, class OpE, typename T, bool VECOK>
+__global__ void __launch_bounds__(kThreads, kGeoMinCtas) suite_geo_kernel(const SuiteGeoArgs g, const Params P) {
+    constexpr int VEC = Vec16<T>::N;
+    constexpr int TILE = kThreads * VEC;
+    constexpr int LU = kGeoLevels;
+#if EK_LEAN_DEVICE
+    if (sizeof(T) == 8) lean::init_tables();
+#endif
+    const int nhalf = g.nlev + 1;
+    coef_smem_fill<T>(static_cast<const T*>(g.A), static_cast<const T*>(g.B), 0, nhalf);
+    const T* sA = coef_smem<T>();
+    const T* sB = sA + nhalf;
+    const T* tq[2] = {static_cast<const T*>(g.t), static_cast<const T*>(g.q)};
+    const int mode = g.mode;
+    const bool want_h = g.height != nullptr;
+    const bool h_zs = want_h && mode != EK_HM_THICKNESS && mode != EK_HM_GH_GROUND;
+    const int form = mode >> 1;  // 0: geopotential units, 1: geopotential height, 2: geometric height
+    const T at = static_cast<T>(g.alpha_top);
+    const int64_t ptiles = (g.npl + TILE - 1) / TILE;
+    for (int64_t pt = blockIdx.x; pt < ptiles; pt += gridDim.x) {
+        const int64_t i0 = pt * TILE + (int64_t)threadIdx.x * VEC;
+        if (i0 >= g.npl) continue;
+        T sp[VEC], zs[VEC], hsub[VEC], sum[VEC], phb[VEC];  // phb: pressure of the half level under the current level
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) zs[j] = hsub[j] = sum[j] = T(0);
+        ld_row<T, VECOK>(static_cast<const T*>(g.sp), i0, g.npl, sp, false);
+        {
+            const T ab = sA[g.nlev], bb = sB[g.nlev];
+#pragma unroll
+            for (int j = 0; j < VEC; ++j) phb[j] = exactm::hyb_half(ab, bb, sp[j]);  // V:663
+        }
+        if (g.z || h_zs) ld_row<T, VECOK>(static_cast<const T*>(g.zs), i0, g.npl, zs, false);
+        if (want_h && mode == EK_HM_GEOM_GROUND) {
+#pragma unroll
+            for (int j = 0; j < VEC; ++j) hsub[j] = EK_FAST_NS::geom_from_z(zs[j]);
+        }
+        for (int k = g.nlev - 1; k >= 0; k -= LU) {
+            T x[LU][2][VEC];
+#pragma unroll
+            for (int u = 0; u < LU; ++u)
+                if (k - u >= 0) {
+#pragma unroll
+                    for (int c = 0; c < 2; ++c) ld_row<T, VECOK>(tq[c] + (int64_t)(k - u) * g.npl, i0, g.npl, x[u][c], true);
+                }
+#pragma unroll
+            for (int u = 0; u < LU; ++u)  // ask L2 for a later group of levels while this group is being computed
+                if (k - LU * kGeoPfDist - u >= 0) {
+#pragma unroll
+                    for (int c = 0; c < 2; ++c) asm volatile("prefetch.global.L2 [%0];" ::"l"(tq[c] + (int64_t)(k - LU * kGeoPfDist - u) * g.npl + i0));
+                }
+#pragma unroll
+            for (int u = 0; u < LU; ++u) {
+                const int kk = k - u;
+                if (kk < 0) break;
+                const T a0 = sA[kk], b0 = sB[kk];
+                const bool top = g.top_toa && kk == 0;
+                T y[S_NSLOTS][VEC], pf[VEC], th[VEC], zz[VEC], hh[VEC];
+#pragma unroll
+                for (int j = 0; j < VEC; ++j) {
+                    const T pht = exactm::hyb_half(a0, b0, sp[j]);  // the half level on top of this level (V:663)
+                    pf[j] = exactm::hyb_full(pht, phb[j]);          // V:708
+                    T de, al;
+                    delta_alpha<T>(pht, phb[j], top, at, de, al);
+                    phb[j] = pht;
+                    T a[3] = {x[u][0][j], x[u][1][j], pf[j]}, r[S_NSLOTS];
+                    point<Op, OpE, T>(a, r, P, 3u);  // t and q are the array inputs; p is derived
+#pragma unroll
+                    for (int o = 0; o < S_NSLOTS; ++o) y[o][j] = r[o];
+                    const T d = exactm::gas_constant(x[u][1][j]) * x[u][0][j];
+                    const T dphi = sum[j] + d * al;  // V:808-809
+                    sum[j] = sum[j] + d * de;        // V:804
+                    th[j] = dphi;
+                    zz[j] = dphi + zs[j];
+                    if (want_h) {
+                        const T z = h_zs ? zz[j] : dphi;
+                        T h = form == 0 ? z : (form == 1 ? EK_FAST_NS::gh_from_z(z) : EK_FAST_NS::geom_from_z(z) - hsub[j]);
+#if EK_LEAN_DEVICE
+                        if (sizeof(T) == 8 && __builtin_expect(is_nan_bits(h), 0)) h = exact_height_output<T>(dphi, zs[j], mode);
+#endif
+                        hh[j] = h;
+                    }
+                }
+                const int64_t off = (int64_t)kk * g.npl;
+#pragma unroll
+                for (int o = 0; o < S_NSLOTS; ++o) {
+                    const bool w = Op::STATIC_MASK ? (((Op::STATIC_MASK >> o) & 1u) != 0) : (g.outs[o] != nullptr);
+                    if (w) st_row<T, VECOK>(static_cast<T*>(g.outs[o]) + off, i0, g.npl, y[o]);
+                }
+                if (g.p_out) st_row<T, VECOK>(static_cast<T*>(g.p_out) + off, i0, g.npl, pf);
+                if (g.thickness) st_row<T, VECOK>(static_cast<T*>(g.thickness) + off, i0, g.npl, th);
+                if (g.z) st_row<T, VECOK>(static_cast<T*>(g.z) + off, i0, g.npl, zz);
+                if (want_h) st_row<T, VECOK>(static_cast<T*>(g.height) + off, i0, g.npl, hh);
+            }
+        }
+    }
+}
+
 int grid_for(int64_t items) {
     const int sms = sm_count_current_device();
     if (sms <= 0) return -1;
@@ -518,22 +640,45 @@ EK_API(geopotential_on_hybrid_levels,
         double alpha_top, const void* alpha, const void* delta, const void* zs, int mode, void* out, void* stream),
        (t, q, nlev, npl, sp, A, B, nhalf, top_toa, alpha_top, alpha, delta, zs, mode, out, stream))
 
+// The suite arguments shared by the hybrid launchers: the ept method (reset to IFS when no slot uses it) and the output table
+// of the requested slots; `vec` is cleared when a buffer is not 16-byte aligned.
+static int suite_outputs(const char* what, void* const* outs, uint32_t out_mask, bool any_other, int& ept_method, void** dst, bool& vec) {
+    if (out_mask >= (1u << S_NSLOTS) || (out_mask == 0 && !any_other)) return set_error(EK_ERR_ARG, "%s: out_mask=0x%x selects no output", what, out_mask);
+    constexpr uint32_t EPT = (1u << S_EPT) | (1u << S_WBPT);
+    if (!(out_mask & EPT)) ept_method = EK_EPT_IFS;
+    if (ept_method < EK_EPT_IFS || ept_method > EK_EPT_BOLTON39) return set_error(EK_ERR_ENUM, "%s: invalid ept method id %d", what, ept_method);
+    for (int k = 0; k < S_NSLOTS; ++k) {
+        dst[k] = ((out_mask >> k) & 1u) ? (outs ? outs[k] : nullptr) : nullptr;
+        if (((out_mask >> k) & 1u) && !dst[k]) return set_error(EK_ERR_ARG, "%s: output %d requested but its buffer is NULL", what, k);
+        vec = vec && ok16(dst[k]);
+    }
+    return EK_OK;
+}
+
+// The suite instantiations of the hybrid kernels: a run-time mask for each non-IFS ept method, and for IFS the two common static
+// masks (the default five outputs, and those with ept + wbpt) or a run-time mask.  LAUNCH(MASK, EPT_METHOD) launches one.
+#define EK_SUITE_DISPATCH(LAUNCH)         \
+    do {                                  \
+        if (ept_method == EK_EPT_BOLTON35) \
+            LAUNCH(0, EPT_BOLTON35);       \
+        else if (ept_method == EK_EPT_BOLTON39) \
+            LAUNCH(0, EPT_BOLTON39);       \
+        else if (out_mask == 0x1F)         \
+            LAUNCH(0x1F, EPT_IFS);         \
+        else if (out_mask == 0x31F)        \
+            LAUNCH(0x31F, EPT_IFS);        \
+        else                               \
+            LAUNCH(0, EPT_IFS);            \
+    } while (0)
+
 template <template <uint32_t, int> class OpM, template <uint32_t, int> class OpME, typename T>
 static int suite_hybrid(const void* t, const void* q, const void* sp, const void* A, const void* B, int nlev, int64_t npl, void* const* outs,
                         uint32_t out_mask, int ept_method, void* p_out, void* stream) {
     const char* what = "suite_tq_hybrid";
     if (!t || !q || !sp || !A || !B || nlev < 1 || npl < 0) return set_error(EK_ERR_ARG, "%s: bad arguments", what);
-    if (out_mask >= (1u << S_NSLOTS) || (out_mask == 0 && !p_out)) return set_error(EK_ERR_ARG, "%s: out_mask=0x%x selects no output", what, out_mask);
-    constexpr uint32_t EPT = (1u << S_EPT) | (1u << S_WBPT);
-    if (!(out_mask & EPT)) ept_method = EK_EPT_IFS;
-    if (ept_method < EK_EPT_IFS || ept_method > EK_EPT_BOLTON39) return set_error(EK_ERR_ENUM, "%s: invalid ept method id %d", what, ept_method);
     SuiteHybridArgs g{t, q, sp, A, B, {}, p_out, nlev, npl, 2};
     bool vec = npl % Vec16<T>::N == 0 && ok16(t) && ok16(q) && ok16(sp) && ok16(p_out);
-    for (int k = 0; k < S_NSLOTS; ++k) {
-        g.outs[k] = ((out_mask >> k) & 1u) ? (outs ? outs[k] : nullptr) : nullptr;
-        if (((out_mask >> k) & 1u) && !g.outs[k]) return set_error(EK_ERR_ARG, "%s: output %d requested but its buffer is NULL", what, k);
-        vec = vec && ok16(g.outs[k]);
-    }
+    if (int rc = suite_outputs(what, outs, out_mask, p_out != nullptr, ept_method, g.outs, vec)) return rc;
     if (npl == 0) return EK_OK;
     constexpr int TILE = kThreads * Vec16<T>::N;
     const int64_t ptiles = (npl + TILE - 1) / TILE;
@@ -553,17 +698,48 @@ static int suite_hybrid(const void* t, const void* q, const void* sp, const void
         else                                                                                                        \
             launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(blocks, st, smem, g, P);    \
     } while (0)
-    if (ept_method == EK_EPT_BOLTON35)
-        EK_LAUNCH_SH(0, EPT_BOLTON35);
-    else if (ept_method == EK_EPT_BOLTON39)
-        EK_LAUNCH_SH(0, EPT_BOLTON39);
-    else if (out_mask == 0x1F)
-        EK_LAUNCH_SH(0x1F, EPT_IFS);
-    else if (out_mask == 0x31F)
-        EK_LAUNCH_SH(0x31F, EPT_IFS);
-    else
-        EK_LAUNCH_SH(0, EPT_IFS);
+    EK_SUITE_DISPATCH(EK_LAUNCH_SH);
 #undef EK_LAUNCH_SH
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
+    return EK_OK;
+}
+
+template <template <uint32_t, int> class OpM, template <uint32_t, int> class OpME, typename T>
+static int suite_hybrid_geo(const void* t, const void* q, const void* sp, const void* zs, const void* A, const void* B, int nlev, int64_t npl,
+                            void* const* outs, uint32_t out_mask, int ept_method, void* p_out, int top_toa, double alpha_top, void* thickness_out,
+                            void* z_out, void* height_out, int height_mode, void* stream) {
+    const char* what = "suite_tq_hybrid_geo";
+    if (!t || !q || !sp || !A || !B || nlev < 1 || npl < 0) return set_error(EK_ERR_ARG, "%s: bad arguments", what);
+    if (height_out && (height_mode < EK_HM_THICKNESS || height_mode > EK_HM_GEOM_GROUND))
+        return set_error(EK_ERR_ENUM, "%s: invalid height mode %d", what, height_mode);
+    const bool need_zs = z_out || (height_out && height_mode != EK_HM_THICKNESS && height_mode != EK_HM_GH_GROUND);
+    if (need_zs && !zs) return set_error(EK_ERR_ARG, "%s: this output needs the surface geopotential zs", what);
+    SuiteGeoArgs g{t, q, sp, need_zs ? zs : nullptr, A, B, {}, p_out, thickness_out, z_out, height_out, nlev, npl, top_toa, alpha_top,
+                   height_out ? height_mode : EK_HM_THICKNESS};
+    bool vec = npl % Vec16<T>::N == 0 && ok16(t) && ok16(q) && ok16(sp) && ok16(g.zs) && ok16(p_out) && ok16(thickness_out) && ok16(z_out) &&
+               ok16(height_out);
+    const bool other = p_out || thickness_out || z_out || height_out;
+    if (int rc = suite_outputs(what, outs, out_mask, other, ept_method, g.outs, vec)) return rc;
+    if (npl == 0) return EK_OK;
+    constexpr int TILE = kThreads * Vec16<T>::N;
+    const int blocks = grid_for((npl + TILE - 1) / TILE);  // one work item per column tile: the level walk is sequential
+    if (blocks < 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
+    Params P;
+    P.out_mask = out_mask;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const unsigned smem = smem_for<T>() + coef_smem_bytes<T>(nlev + 1);  // lean tables (float64) + the half-level coefficients
+    if (smem > 200u * 1024u) return set_error(EK_ERR_ARG, "%s: nlev=%d is too large for the shared-memory coefficient copy", what, nlev);
+#define EK_LAUNCH_SG(M, EM)                                                                                       \
+    do {                                                                                                          \
+        if (vec)                                                                                                  \
+            launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(blocks, st, smem, g, P);      \
+        else                                                                                                      \
+            launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(blocks, st, smem, g, P);     \
+    } while (0)
+    EK_SUITE_DISPATCH(EK_LAUNCH_SG);
+#undef EK_LAUNCH_SG
     g_launches.fetch_add(1, std::memory_order_relaxed);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
@@ -580,6 +756,19 @@ EK_API(suite_tq_hybrid,
         int ept_method, void* p_out, void* stream),
        (t, q, sp, A, B, nlev, npl, outs, out_mask, ept_method, p_out, stream))
 
+template <typename T>
+static int impl_suite_tq_hybrid_geo(const void* t, const void* q, const void* sp, const void* zs, const void* A, const void* B, int nlev, int64_t npl,
+                                    void* const* outs, uint32_t out_mask, int ept_method, void* p_out, int top_toa, double alpha_top,
+                                    void* thickness_out, void* z_out, void* height_out, int height_mode, void* stream) {
+    return suite_hybrid_geo<EK_OPS(OpSuiteTQPm), T>(t, q, sp, zs, A, B, nlev, npl, outs, out_mask, ept_method, p_out, top_toa, alpha_top, thickness_out,
+                                                    z_out, height_out, height_mode, stream);
+}
+EK_API(suite_tq_hybrid_geo,
+       (const void* t, const void* q, const void* sp, const void* zs, const void* A, const void* B, int nlev, int64_t npl, void* const* outs,
+        uint32_t out_mask, int ept_method, void* p_out, int top_toa, double alpha_top, void* thickness_out, void* z_out, void* height_out,
+        int height_mode, void* stream),
+       (t, q, sp, zs, A, B, nlev, npl, outs, out_mask, ept_method, p_out, top_toa, alpha_top, thickness_out, z_out, height_out, height_mode, stream))
+
 // used by the host-buffer pipeline in ek_api.cu
 template <typename T>
 int ek_suite_launch_hybrid(const void* t, const void* q, const void* sp, const void* A, const void* B, int nlev, int64_t npl, void* const* outs,
@@ -588,3 +777,14 @@ int ek_suite_launch_hybrid(const void* t, const void* q, const void* sp, const v
 }
 template int ek_suite_launch_hybrid<double>(const void*, const void*, const void*, const void*, const void*, int, int64_t, void* const*, uint32_t, int, void*);
 template int ek_suite_launch_hybrid<float>(const void*, const void*, const void*, const void*, const void*, int, int64_t, void* const*, uint32_t, int, void*);
+template <typename T>
+int ek_suite_launch_hybrid_geo(const void* t, const void* q, const void* sp, const void* zs, const void* A, const void* B, int nlev, int64_t npl,
+                               void* const* outs, uint32_t out_mask, int ept_method, int top_toa, double alpha_top, void* const* cols,
+                               int height_mode, void* stream) {
+    return suite_hybrid_geo<EK_OPS(OpSuiteTQPm), T>(t, q, sp, zs, A, B, nlev, npl, outs, out_mask, ept_method, nullptr, top_toa, alpha_top, cols[0],
+                                                    cols[1], cols[2], height_mode, stream);
+}
+template int ek_suite_launch_hybrid_geo<double>(const void*, const void*, const void*, const void*, const void*, const void*, int, int64_t,
+                                                void* const*, uint32_t, int, int, double, void* const*, int, void*);
+template int ek_suite_launch_hybrid_geo<float>(const void*, const void*, const void*, const void*, const void*, const void*, int, int64_t,
+                                               void* const*, uint32_t, int, int, double, void* const*, int, void*);

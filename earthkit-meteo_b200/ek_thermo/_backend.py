@@ -127,6 +127,10 @@ for _sfx in ("f64", "f32"):
     _fn.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, ctypes.POINTER(c_void_p), c_uint32, c_int, c_void_p,
                     c_void_p]
     _fn.restype = c_int
+    _fn = getattr(_lib, f"ek_thermo_suite_tq_hybrid_geo_{_sfx}")
+    _fn.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, ctypes.POINTER(c_void_p), c_uint32, c_int, c_void_p,
+                    c_int, c_double, c_void_p, c_void_p, c_void_p, c_int, c_void_p]
+    _fn.restype = c_int
 for _sfx in ("f64", "f32"):
     _fn = getattr(_lib, f"ek_thermo_host_suite_{_sfx}")
     _fn.argtypes = [c_int, c_void_p, c_void_p, c_void_p, ctypes.POINTER(c_void_p), c_uint32, c_int, c_int64, c_void_p, c_size_t, c_int]
@@ -134,6 +138,10 @@ for _sfx in ("f64", "f32"):
     _fn = getattr(_lib, f"ek_thermo_host_suite_tq_hybrid_{_sfx}")
     _fn.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, ctypes.POINTER(c_void_p), c_uint32, c_int, c_void_p,
                     c_size_t, c_int]
+    _fn.restype = c_int
+    _fn = getattr(_lib, f"ek_thermo_host_suite_tq_hybrid_geo_{_sfx}")
+    _fn.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, ctypes.POINTER(c_void_p), c_uint32, c_int, c_int,
+                    c_double, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_int]
     _fn.restype = c_int
 
 
@@ -460,4 +468,17 @@ def host_suite_tq_hybrid(dtype, h_t, h_q, h_sp, h_a, h_b, nlev: int, npl: int, h
         torch.cuda.current_stream().synchronize()
         _check(fn(c_void_p(h_t), c_void_p(h_q), c_void_p(h_sp), c_void_p(h_a), c_void_p(h_b), c_int(nlev), c_int64(npl),
                   ctypes.cast(outs, ctypes.POINTER(c_void_p)), c_uint32(mask), c_int(ept_method), c_void_p(workspace.data_ptr()),
+                  c_size_t(workspace.numel() * workspace.element_size()), c_int(n_slots)))
+
+
+def host_suite_tq_hybrid_geo(dtype, h_t, h_q, h_sp, h_zs, h_a, h_b, nlev: int, npl: int, h_out_ptrs, mask: int, ept_method: int, top_toa: int,
+                             alpha_top: float, h_cols, height_mode: int, workspace: torch.Tensor, n_slots: int):
+    """``h_cols``: host pointers (or None) of the thickness, z and height outputs."""
+    fn = getattr(_lib, f"ek_thermo_host_suite_tq_hybrid_geo_{_SUFFIX[dtype]}")
+    outs = (c_void_p * N_SUITE_SLOTS)(*h_out_ptrs)
+    with torch.cuda.device(workspace.device):
+        torch.cuda.current_stream().synchronize()
+        _check(fn(c_void_p(h_t), c_void_p(h_q), c_void_p(h_sp), c_void_p(h_zs), c_void_p(h_a), c_void_p(h_b), c_int(nlev), c_int64(npl),
+                  ctypes.cast(outs, ctypes.POINTER(c_void_p)), c_uint32(mask), c_int(ept_method), c_int(top_toa), c_double(alpha_top),
+                  *(c_void_p(p) for p in h_cols), c_int(height_mode), c_void_p(workspace.data_ptr()),
                   c_size_t(workspace.numel() * workspace.element_size()), c_int(n_slots)))

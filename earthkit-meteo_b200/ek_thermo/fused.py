@@ -7,6 +7,8 @@ named in ``SUITE_TQP_OUTPUTS`` / ``SUITE_TTDP_OUTPUTS`` applied to the same inpu
 """
 from __future__ import annotations
 
+import math
+
 from . import _backend as _b
 
 # output name -> slot (include/ek_thermo.h EK_S_*), with the reference function each one equals
@@ -90,7 +92,34 @@ def suite_ttdp_batch(ts, tds, ps, outputs=DEFAULT_TTDP, out=None, ept_method="if
     return _b.execute_suite_batch("suite_ttdp_batch", (ts, tds, ps), outputs, _slots(SUITE_TTDP_OUTPUTS, outputs), out, _ept_id(ept_method))
 
 
-def suite_tq_hybrid(t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, want_p=False, ept_method="ifs"):
+# column outputs of suite_tq_hybrid: the geopotential of the same levels, from the same walk of the columns
+COLUMN_OUTPUTS = (
+    "thickness",  # relative_geopotential_thickness_on_hybrid_levels(t, q, A, B, sp, alpha_top)                      V:894-994
+    "z",  # geopotential_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top)                                            V:997-1069
+    "height",  # height_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top, h_type, h_reference)                        V:1072-1188
+)
+# Fields of fewer columns than this run a mixed call as the suite launch plus one geopotential_on_hybrid_levels launch per column
+# output: the fused walk has one work item per tile of 256 threads x one 16-byte vector of columns (512 columns in float64, 1024 in
+# float32), so a small field leaves most of the GPU idle, while the suite launch also splits the levels into work items.  Measured
+# on B200, 5 outputs + z x 137 levels, fused / two launches (profiles/r03_kbench_geo_*.log): float64 0.91 at 65 536 columns, 1.20 at
+# 32 768; float32 0.81 at 262 144, 1.05 at 131 072.
+GEO_FUSED_MIN_COLUMNS = {"float64": 65536, "float32": 262144}
+
+
+def _out_buffer(out, name, like):
+    """out[name] when the caller preallocated it (checked), else a new tensor like `like`."""
+    import torch
+
+    if out is not None and name in out:
+        o = out[name]
+        if o.dtype != like.dtype or o.shape != like.shape or not o.is_contiguous() or o.device != like.device:
+            raise ValueError(f"suite_tq_hybrid: preallocated output {name!r} must be a contiguous {like.dtype} tensor of shape {tuple(like.shape)}")
+        return o
+    return torch.empty_like(like)
+
+
+def suite_tq_hybrid(t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, want_p=False, ept_method="ifs", zs=None, alpha_top="ifs", h_type="geometric",
+                    h_reference="ground"):
     """The (t, q, p) suite on hybrid model levels with the pressure computed inside the kernel.
 
     ``t`` and ``q`` are ``[nlev, ...]`` fields, ``sp`` the surface pressure ``[...]``, ``A`` / ``B`` the ``nlev + 1``
@@ -98,14 +127,31 @@ def suite_tq_hybrid(t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, want_p=False,
     ``p = earthkit.meteo.vertical.pressure_on_hybrid_levels(A, B, sp, output="full")`` (reference
     vertical/array/vertical.py:663,708) -- but the ``[nlev, ...]`` pressure array is never written or read:
     56 instead of 64 bytes per point for the five default outputs.  ``want_p=True`` also returns it (key ``"p"``).
+
+    ``outputs`` may also name the column outputs of ``COLUMN_OUTPUTS``, the geopotential of the same levels:
+    ``"thickness"`` (``relative_geopotential_thickness_on_hybrid_levels``), ``"z"`` (``geopotential_on_hybrid_levels``) and
+    ``"height"`` (``height_on_hybrid_levels`` with ``h_type`` / ``h_reference``: "geometric" or any other h_type for
+    geopotential height, "ground" or "sea"), all with ``alpha_top`` ("ifs" / "arpege").  ``zs``, the surface geopotential (a
+    tensor of ``sp.shape`` or a Python number), is needed by ``"z"`` and by every height except geopotential height above
+    ground.  With suite outputs too, one kernel walks the columns and reads ``t`` and ``q`` once for both (64 instead of 80
+    bytes per point for five suite outputs and ``"z"`` in float64).  The column outputs have the dtype of the field: they equal
+    the ``ek_thermo.vertical`` functions called with ``A`` / ``B`` given as tensors of that dtype (not the float64 promotion
+    those functions apply to Python-list ``A`` / ``B``).
     """
     import ctypes
-    from ctypes import c_int, c_int64, c_uint32, c_void_p
+    from ctypes import c_double, c_int, c_int64, c_uint32, c_void_p
 
     import torch
 
+    from .vertical import _column_kernel, _height_mode, _top_is_toa
+
     outputs = tuple(outputs)
-    slots = _slots(SUITE_TQP_OUTPUTS, outputs)
+    cols = tuple(o for o in outputs if o in COLUMN_OUTPUTS)
+    suite = tuple(o for o in outputs if o not in COLUMN_OUTPUTS)
+    slots = _slots(SUITE_TQP_OUTPUTS, suite)
+    if alpha_top not in ("ifs", "arpege"):
+        raise ValueError(f"Unknown method '{alpha_top}' for pressure calculation. Use 'ifs' or 'arpege'.")
+    hmode = _height_mode(h_type, h_reference)
     for x in (t, q, sp):
         if not isinstance(x, torch.Tensor):
             raise TypeError("suite_tq_hybrid: t, q and sp must be torch CUDA tensors")
@@ -120,35 +166,51 @@ def suite_tq_hybrid(t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, want_p=False,
     b = torch.as_tensor(B, dtype=dtype, device=dev).contiguous()
     if a.numel() != nlev + 1 or b.numel() != nlev + 1:
         raise ValueError(f"suite_tq_hybrid: A and B need nlev + 1 = {nlev + 1} half-level values")
+    modes = {"thickness": 0, "z": 1, "height": hmode}
+    if any(modes[c] not in (0, 3) for c in cols):
+        if zs is None:
+            raise ValueError("suite_tq_hybrid: 'z' and every 'height' except geopotential height above ground need the surface geopotential zs")
+        if isinstance(zs, torch.Tensor):
+            _b._check_device([t, zs])
+            if zs.dtype != dtype or zs.shape != sp.shape:
+                raise ValueError(f"suite_tq_hybrid: zs must be a {dtype} tensor of shape {tuple(sp.shape)} or a Python number")
+        elif not isinstance(zs, (int, float)) or isinstance(zs, bool):
+            raise TypeError("suite_tq_hybrid: zs must be a torch CUDA tensor or a Python number")
+    else:
+        zs = None
     tc, qc, spc = t.contiguous(), q.contiguous(), sp.contiguous()
     ptrs = (c_void_p * _b.N_SUITE_SLOTS)()
     mask = 0
     res = {}
     em = _ept_id(ept_method)
-    for name, k in zip(outputs, slots):
-        if out is not None and name in out:
-            o = out[name]
-            if o.dtype != dtype or o.shape != t.shape or not o.is_contiguous() or o.device != dev:
-                raise ValueError(f"suite_tq_hybrid: preallocated output {name!r} must be a contiguous {dtype} tensor of shape {tuple(t.shape)}")
-        else:
-            o = torch.empty_like(tc)
-        res[name] = o
-        ptrs[k] = o.data_ptr()
+    for name in outputs:
+        res[name] = _out_buffer(out, name, tc)
+    for name, k in zip(suite, slots):
+        ptrs[k] = res[name].data_ptr()
         mask |= 1 << k
     p_ptr = c_void_p(None)
     if want_p:
-        if out is not None and "p" in out:
-            o = out["p"]
-            if o.dtype != dtype or o.shape != t.shape or not o.is_contiguous() or o.device != dev:
-                raise ValueError(f"suite_tq_hybrid: preallocated output 'p' must be a contiguous {dtype} tensor of shape {tuple(t.shape)}")
-            res["p"] = o
-        else:
-            res["p"] = torch.empty_like(tc)
+        res["p"] = _out_buffer(out, "p", tc)
         p_ptr = c_void_p(res["p"].data_ptr())
-    if npl > 0:
+    if npl == 0:
+        return res
+    fused = bool(cols) and (bool(suite) or want_p) and npl >= GEO_FUSED_MIN_COLUMNS["float64" if dtype == torch.float64 else "float32"]
+    if not fused and (suite or want_p or not cols):
         _b.call_raw("suite_tq_hybrid", dtype, dev, c_void_p(tc.data_ptr()), c_void_p(qc.data_ptr()), c_void_p(spc.data_ptr()),
                     c_void_p(a.data_ptr()), c_void_p(b.data_ptr()), c_int(nlev), c_int64(npl), ctypes.cast(ptrs, ctypes.POINTER(c_void_p)),
                     c_uint32(mask), c_int(em), p_ptr)
+    if not fused:
+        for name in cols:
+            _column_kernel(tc, qc, modes[name], 0, sp=spc, A=a, B=b, alpha_top=alpha_top, zs=zs, out=res[name])
+        return res
+    zsc = None
+    if zs is not None:
+        zsc = zs.contiguous() if isinstance(zs, torch.Tensor) else torch.full(tuple(sp.shape), float(zs), dtype=dtype, device=dev)
+    col_ptr = lambda n: c_void_p(res[n].data_ptr()) if n in res else c_void_p(None)  # noqa: E731
+    _b.call_raw("suite_tq_hybrid_geo", dtype, dev, c_void_p(tc.data_ptr()), c_void_p(qc.data_ptr()), c_void_p(spc.data_ptr()),
+                c_void_p(zsc.data_ptr() if zsc is not None else None), c_void_p(a.data_ptr()), c_void_p(b.data_ptr()), c_int(nlev), c_int64(npl),
+                ctypes.cast(ptrs, ctypes.POINTER(c_void_p)), c_uint32(mask), c_int(em), p_ptr, c_int(_top_is_toa(a, b, 0, spc, dtype, dev)),
+                c_double(math.log(2.0) if alpha_top == "ifs" else 1.0), col_ptr("thickness"), col_ptr("z"), col_ptr("height"), c_int(hmode))
     return res
 
 

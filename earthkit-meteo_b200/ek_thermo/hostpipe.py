@@ -6,11 +6,13 @@ several streams (ek_thermo_host_suite_*).  All arithmetic still happens on the G
 """
 from __future__ import annotations
 
+import math
+
 import numpy as np
 import torch
 
 from . import _backend as _b
-from .fused import DEFAULT_TQP, DEFAULT_TTDP, SUITE_TQP_OUTPUTS, SUITE_TTDP_OUTPUTS
+from .fused import COLUMN_OUTPUTS, DEFAULT_TQP, DEFAULT_TTDP, SUITE_TQP_OUTPUTS, SUITE_TTDP_OUTPUTS
 
 _TORCH = {np.dtype("float64"): torch.float64, np.dtype("float32"): torch.float32}
 
@@ -98,9 +100,20 @@ class HostSuite:
     def suite_ttdp(self, t, td, p, outputs=DEFAULT_TTDP, out=None, ept_method="ifs"):
         return self._run(1, SUITE_TTDP_OUTPUTS, t, td, p, tuple(outputs), out, ept_method)
 
-    def suite_tq_hybrid(self, t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, ept_method="ifs"):
+    def suite_tq_hybrid(self, t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, ept_method="ifs", zs=None, alpha_top="ifs", h_type="geometric",
+                        h_reference="ground"):
         """``fused.suite_tq_hybrid`` for host arrays: t, q ``[nlev, npl]``, sp ``[npl]``, A / B ``nlev + 1`` half-level values.
-        The pressure field crosses PCIe in neither direction (sp travels instead: 16 + 8/nlev bytes per point in)."""
+        The pressure field crosses PCIe in neither direction (sp travels instead: 16 + 8/nlev bytes per point in).  The column
+        outputs ``"thickness"``, ``"z"`` and ``"height"`` with ``zs`` (a ``[npl]`` array or a Python number), ``alpha_top``,
+        ``h_type`` and ``h_reference`` as there; they come from the same kernel pass over each chunk."""
+        from .vertical import _height_mode, _top_is_toa
+
+        outputs = tuple(outputs)
+        cols = tuple(o for o in outputs if o in COLUMN_OUTPUTS)
+        suite = tuple(o for o in outputs if o not in COLUMN_OUTPUTS)
+        if alpha_top not in ("ifs", "arpege"):
+            raise ValueError(f"Unknown method '{alpha_top}' for pressure calculation. Use 'ifs' or 'arpege'.")
+        hmode = _height_mode(h_type, h_reference)
         t, q, sp = (np.ascontiguousarray(x) for x in (t, q, sp))
         dt = t.dtype
         if dt not in _TORCH or q.dtype != dt or sp.dtype != dt or t.ndim != 2 or q.shape != t.shape or sp.shape != t.shape[1:]:
@@ -110,7 +123,24 @@ class HostSuite:
         b = np.ascontiguousarray(np.asarray(B, dtype=dt))
         if a.shape != (nlev + 1,) or b.shape != (nlev + 1,):
             raise ValueError(f"host suite: A and B need nlev + 1 = {nlev + 1} half-level values")
-        res, ptrs, mask = self._outputs(SUITE_TQP_OUTPUTS, tuple(outputs), out, t.shape, dt)
-        _b.host_suite_tq_hybrid(_TORCH[dt], t.ctypes.data, q.ctypes.data, sp.ctypes.data, a.ctypes.data, b.ctypes.data, nlev, npl, ptrs, mask,
-                                _EPT[ept_method], self.workspace, self.n_slots)
+        res, ptrs, mask = self._outputs(SUITE_TQP_OUTPUTS, suite, out, t.shape, dt)
+        if not cols:
+            _b.host_suite_tq_hybrid(_TORCH[dt], t.ctypes.data, q.ctypes.data, sp.ctypes.data, a.ctypes.data, b.ctypes.data, nlev, npl, ptrs, mask,
+                                    _EPT[ept_method], self.workspace, self.n_slots)
+            return res
+        modes = {"thickness": 0, "z": 1, "height": hmode}
+        zs_ptr = None
+        if any(modes[c] not in (0, 3) for c in cols):
+            if zs is None:
+                raise ValueError("host suite: 'z' and every 'height' except geopotential height above ground need the surface geopotential zs")
+            zs = np.full(sp.shape, zs, dtype=dt) if isinstance(zs, (int, float)) and not isinstance(zs, bool) else np.ascontiguousarray(zs)
+            if zs.dtype != dt or zs.shape != sp.shape:
+                raise TypeError(f"host suite: zs must be a {dt} array of shape {sp.shape} or a Python number")
+            zs_ptr = zs.ctypes.data
+        col_res, _, _ = self._outputs({c: 0 for c in cols}, cols, out, t.shape, dt)
+        res.update(col_res)
+        res = {name: res[name] for name in outputs}
+        _b.host_suite_tq_hybrid_geo(_TORCH[dt], t.ctypes.data, q.ctypes.data, sp.ctypes.data, zs_ptr, a.ctypes.data, b.ctypes.data, nlev, npl, ptrs,
+                                    mask, _EPT[ept_method], _top_is_toa(a, b, 0, sp, None, None), math.log(2.0) if alpha_top == "ifs" else 1.0,
+                                    [res[c].ctypes.data if c in res else None for c in COLUMN_OUTPUTS], hmode, self.workspace, self.n_slots)
         return res

@@ -9,6 +9,7 @@ from __future__ import annotations
 import math
 from ctypes import c_double, c_int, c_int64, c_void_p
 
+import numpy as np
 import torch
 
 from . import _backend as _b
@@ -56,10 +57,14 @@ def _coeff_tensors(A, B, dtype, device):
 
 
 def _top_is_toa(a, b, top_half, spc, dtype, dev):
-    """V:678: does ANY point have p_half[top] <= 0.1 Pa?  A constant when B[top] == 0, else a one-flag reduction kernel."""
+    """V:678: does ANY point have p_half[top] <= 0.1 Pa?  A constant when B[top] == 0, else a one-flag reduction kernel -- or, for
+    a host (numpy) ``spc`` with ``a`` / ``b`` of its dtype, the same comparison on the host."""
     a_top, b_top = float(a[top_half]), float(b[top_half])
-    if b_top == 0.0 or spc.numel() == 0:
+    host = isinstance(spc, np.ndarray)
+    if b_top == 0.0 or (spc.size if host else spc.numel()) == 0:
         return int(a_top <= 0.1)
+    if host:
+        return int(np.any(a[top_half] + b[top_half] * spc <= spc.dtype.type(0.1)))
     flag = torch.zeros(1, dtype=torch.int32, device=dev)
     _b.call_raw("hybrid_top_is_toa", dtype, dev, c_void_p(spc.data_ptr()), c_int64(spc.numel()), c_double(a_top), c_double(b_top),
                 c_void_p(flag.data_ptr()))
@@ -134,7 +139,7 @@ _HM = {"thickness": 0, "geopotential": 1, ("geopotential", "sea"): 2, ("geopoten
        ("geometric", "ground"): 5}
 
 
-def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top="ifs", alpha=None, delta=None, zs=None):
+def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top="ifs", alpha=None, delta=None, zs=None, out=None):
     for x in (t, q):
         if not isinstance(x, torch.Tensor):
             raise TypeError("ek_thermo.vertical: t and q must be torch CUDA tensors (no CPU path)")
@@ -185,7 +190,8 @@ def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top
         top_toa = _top_is_toa(a, b, nhalf - 1 - nlev, keep[-1], dtype, dev)  # the band is the nlev bottom-most levels (V:1191-1203)
     if mode in (1, 2, 4, 5):
         p_zs = col(zs, "zs")
-    out = torch.empty_like(tc)
+    if out is None:
+        out = torch.empty_like(tc)
     if npl > 0 and nlev > 0:
         _b.call_raw("geopotential_on_hybrid_levels", dtype, dev, c_void_p(tc.data_ptr()), c_void_p(qc.data_ptr()), c_int(nlev), c_int64(npl),
                     p_sp, p_a, p_b, c_int(nhalf), c_int(top_toa), c_double(math.log(2.0) if alpha_top == "ifs" else 1.0), p_al, p_de, p_zs,
@@ -251,11 +257,16 @@ def geopotential_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top="ifs", vertical_
     return _column_kernel(t, q, 1, vertical_axis, sp=sp, A=A, B=B, alpha_top=alpha_top, zs=zs)
 
 
-def height_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top="ifs", h_type="geometric", h_reference="ground", vertical_axis=0):
-    """Geometric / geopotential height above sea level / ground, one kernel.  Reference V:1072-1188."""
+def _height_mode(h_type, h_reference):
+    """The EK_HM_* form of height_on_hybrid_levels' h_type / h_reference (V:1163-1188)."""
     if h_reference not in ["sea", "ground"]:
         raise ValueError(f"Unknown '{h_reference=}'. Use 'sea' or 'ground'.")  # V:1163-1164
-    mode = _HM[("geometric" if h_type == "geometric" else "geopotential", h_reference)]  # any other h_type -> geopotential (V:1175-1186)
+    return _HM[("geometric" if h_type == "geometric" else "geopotential", h_reference)]  # any other h_type -> geopotential (V:1175-1186)
+
+
+def height_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top="ifs", h_type="geometric", h_reference="ground", vertical_axis=0):
+    """Geometric / geopotential height above sea level / ground, one kernel.  Reference V:1072-1188."""
+    mode = _height_mode(h_type, h_reference)
     if vertical_axis != 0:
         return _height_form(_thickness_axis_as_reference(t, q, A, B, sp, alpha_top, vertical_axis), zs, mode)
     return _column_kernel(t, q, mode, vertical_axis, sp=sp, A=A, B=B, alpha_top=alpha_top, zs=zs)

@@ -30,8 +30,9 @@
 extern "C" {
 #endif
 
-#define EK_THERMO_VERSION 111 /* 0.1.1: suite slots 8 (ept) / 9 (wbpt) and their ept_method argument; host pipelines for every suite;
-                                  batched suites with one pressure per level */
+#define EK_THERMO_VERSION 112 /* 0.1.2: the hybrid-level suite with geopotential / height of the same levels in one pass
+                                  (suite_tq_hybrid_geo, host_suite_tq_hybrid_geo).  0.1.1: suite slots 8 (ept) / 9 (wbpt) and their
+                                  ept_method argument; host pipelines for every suite; batched suites with one pressure per level */
 
 typedef struct ek_operand {
     const void* ptr; /* device pointer, or NULL for a broadcast scalar */
@@ -200,6 +201,20 @@ EK_THERMO_FN(height_from_thickness, ek_operand dphi, ek_operand zs, int mode, vo
  * t, q and every output are [nlev, npl]; p_out (optional) receives the pressure itself */
 EK_THERMO_FN(suite_tq_hybrid, const void* t, const void* q, const void* sp, const void* A, const void* B, int nlev, int64_t npl,
              void* const* outs, uint32_t out_mask, int ept_method, void* p_out, void* stream)
+/* suite_tq_hybrid and the geopotential of the same levels in one walk of the columns (bottom to top): t and q are read once
+ * for both.  t, q, outs, out_mask, ept_method, p_out as for suite_tq_hybrid (the suite: T:801-829 ... T:1637-1675 at the
+ * slots of EK_S_*; p: V:663,708); out_mask may be 0 when a column output is given.  The column outputs are
+ * geopotential_on_hybrid_levels over all nlev levels (A, B: nlev + 1 half-level coefficients), any may be NULL:
+ *   thickness_out  dphi, relative_geopotential_thickness_on_hybrid_levels (V:894-994; d = R(q) t, V:799-810);
+ *   z_out          dphi + zs, geopotential_on_hybrid_levels (V:997-1069);
+ *   height_out     form height_mode (EK_HM_*) of dphi, height_on_hybrid_levels (V:1072-1188).
+ * zs: surface geopotential [npl], needed by z_out and by the height modes that add it (all but EK_HM_THICKNESS and
+ * EK_HM_GH_GROUND), else may be NULL.  top_toa: any(A[0] + B[0] * sp <= 0.1) over the field (V:678; ek_thermo_hybrid_top_is_toa
+ * computes it); alpha_top = ln 2 ("ifs") or 1.0 ("arpege") (V:669).  Every output is bit-identical to the separate
+ * suite_tq_hybrid and geopotential_on_hybrid_levels launches on the same arrays. */
+EK_THERMO_FN(suite_tq_hybrid_geo, const void* t, const void* q, const void* sp, const void* zs, const void* A, const void* B, int nlev,
+             int64_t npl, void* const* outs, uint32_t out_mask, int ept_method, void* p_out, int top_toa, double alpha_top,
+             void* thickness_out, void* z_out, void* height_out, int height_mode, void* stream)
 
 /* ---- host-buffer pipelines: the same suite kernels fed from HOST arrays ------------------------------
  * Stream n points through the GPU in chunks: H2D copy, kernel and D2H copy of successive chunks overlap on
@@ -215,6 +230,12 @@ EK_THERMO_FN(host_suite, int kind, const void* h_a, const void* h_b, const void*
  * to the device).  Chunks are column ranges of all levels, moved as 2-D copies. */
 EK_THERMO_FN(host_suite_tq_hybrid, const void* h_t, const void* h_q, const void* h_sp, const void* h_A, const void* h_B, int nlev,
              int64_t npl, void* const* h_outs, uint32_t out_mask, int ept_method, void* workspace, size_t workspace_bytes, int n_slots)
+/* suite_tq_hybrid_geo from HOST arrays: h_t, h_q, every suite output and h_thickness / h_z / h_height [nlev, npl], h_sp and h_zs
+ * [npl], h_A / h_B nlev + 1 half-level coefficients; zs, top_toa, alpha_top, height_mode and the NULL rules as for
+ * suite_tq_hybrid_geo (no pressure output).  h_zs travels with each chunk only when an output needs it. */
+EK_THERMO_FN(host_suite_tq_hybrid_geo, const void* h_t, const void* h_q, const void* h_sp, const void* h_zs, const void* h_A, const void* h_B,
+             int nlev, int64_t npl, void* const* h_outs, uint32_t out_mask, int ept_method, int top_toa, double alpha_top, void* h_thickness,
+             void* h_z, void* h_height, int height_mode, void* workspace, size_t workspace_bytes, int n_slots)
 
 #ifdef __cplusplus
 }
