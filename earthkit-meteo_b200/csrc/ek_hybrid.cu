@@ -568,10 +568,9 @@ static int impl_pressure_on_hybrid_levels(const void* A, const void* B, int nhal
     if (blocks < 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
     const bool vec = npl % Vec16<T>::N == 0 && ok16(sp) && ok16(full) && ok16(half) && ok16(delta) && ok16(alpha);
     const unsigned smem = (delta || alpha) ? smem_for<T>() : 0u;  // the log table, for delta / alpha only
-    if (vec)
-        launch_kernel_smem<&hybrid_pressure_kernel<T, true>>(blocks, static_cast<cudaStream_t>(stream), smem, g);
-    else
-        launch_kernel_smem<&hybrid_pressure_kernel<T, false>>(blocks, static_cast<cudaStream_t>(stream), smem, g);
+    const int rc = vec ? launch_kernel_smem<&hybrid_pressure_kernel<T, true>>(blocks, static_cast<cudaStream_t>(stream), smem, g)
+                       : launch_kernel_smem<&hybrid_pressure_kernel<T, false>>(blocks, static_cast<cudaStream_t>(stream), smem, g);
+    if (rc) return rc;
     g_launches.fetch_add(1, std::memory_order_relaxed);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
@@ -615,21 +614,23 @@ static int impl_geopotential_on_hybrid_levels(const void* t, const void* q, int 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const unsigned smem = smem_for<T>() + (given ? 0u : coef_smem_bytes<T>(nlev + 1));  // lean tables + the band's half-level coefficients
     if (smem > 200u * 1024u) return set_error(EK_ERR_ARG, "%s: nlev=%d is too large for the shared-memory coefficient copy", what, nlev);
+    int rc;
     if (given) {
-        if (vec) launch_kernel_smem<&column_geopotential_kernel<T, true, true, -1>>(blocks, st, smem, g);
-        else launch_kernel_smem<&column_geopotential_kernel<T, true, false, -1>>(blocks, st, smem, g);
+        if (vec) rc = launch_kernel_smem<&column_geopotential_kernel<T, true, true, -1>>(blocks, st, smem, g);
+        else rc = launch_kernel_smem<&column_geopotential_kernel<T, true, false, -1>>(blocks, st, smem, g);
     } else if (!vec) {
-        launch_kernel_smem<&column_geopotential_kernel<T, false, false, -1>>(blocks, st, smem, g);
+        rc = launch_kernel_smem<&column_geopotential_kernel<T, false, false, -1>>(blocks, st, smem, g);
     } else {  // the whole-field case: one instantiation per output form
         switch (mode) {
-            case EK_HM_THICKNESS: launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_THICKNESS>>(blocks, st, smem, g); break;
-            case EK_HM_GEOPOTENTIAL: launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOPOTENTIAL>>(blocks, st, smem, g); break;
-            case EK_HM_GH_SEA: launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GH_SEA>>(blocks, st, smem, g); break;
-            case EK_HM_GH_GROUND: launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GH_GROUND>>(blocks, st, smem, g); break;
-            case EK_HM_GEOM_SEA: launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOM_SEA>>(blocks, st, smem, g); break;
-            default: launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOM_GROUND>>(blocks, st, smem, g); break;
+            case EK_HM_THICKNESS: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_THICKNESS>>(blocks, st, smem, g); break;
+            case EK_HM_GEOPOTENTIAL: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOPOTENTIAL>>(blocks, st, smem, g); break;
+            case EK_HM_GH_SEA: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GH_SEA>>(blocks, st, smem, g); break;
+            case EK_HM_GH_GROUND: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GH_GROUND>>(blocks, st, smem, g); break;
+            case EK_HM_GEOM_SEA: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOM_SEA>>(blocks, st, smem, g); break;
+            default: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOM_GROUND>>(blocks, st, smem, g); break;
         }
     }
+    if (rc) return rc;
     g_launches.fetch_add(1, std::memory_order_relaxed);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
@@ -691,14 +692,16 @@ static int suite_hybrid(const void* t, const void* q, const void* sp, const void
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const unsigned smem = smem_for<T>() + coef_smem_bytes<T>(nlev + 1);  // lean tables (float64) + the half-level coefficients
     if (smem > 200u * 1024u) return set_error(EK_ERR_ARG, "%s: nlev=%d is too large for the shared-memory coefficient copy", what, nlev);
-#define EK_LAUNCH_SH(M, EM)                                                                                         \
-    do {                                                                                                            \
-        if (vec)                                                                                                    \
-            launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(blocks, st, smem, g, P);     \
-        else                                                                                                        \
-            launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(blocks, st, smem, g, P);    \
+#define EK_LAUNCH_SH(M, EM)                                                                                      \
+    do {                                                                                                         \
+        if (vec)                                                                                                 \
+            rc = launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(blocks, st, smem, g, P); \
+        else                                                                                                     \
+            rc = launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(blocks, st, smem, g, P); \
     } while (0)
+    int rc;
     EK_SUITE_DISPATCH(EK_LAUNCH_SH);
+    if (rc) return rc;
 #undef EK_LAUNCH_SH
     g_launches.fetch_add(1, std::memory_order_relaxed);
     cudaError_t err = cudaGetLastError();
@@ -731,14 +734,16 @@ static int suite_hybrid_geo(const void* t, const void* q, const void* sp, const 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const unsigned smem = smem_for<T>() + coef_smem_bytes<T>(nlev + 1);  // lean tables (float64) + the half-level coefficients
     if (smem > 200u * 1024u) return set_error(EK_ERR_ARG, "%s: nlev=%d is too large for the shared-memory coefficient copy", what, nlev);
-#define EK_LAUNCH_SG(M, EM)                                                                                       \
-    do {                                                                                                          \
-        if (vec)                                                                                                  \
-            launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(blocks, st, smem, g, P);      \
-        else                                                                                                      \
-            launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(blocks, st, smem, g, P);     \
+#define EK_LAUNCH_SG(M, EM)                                                                                      \
+    do {                                                                                                         \
+        if (vec)                                                                                                 \
+            rc = launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(blocks, st, smem, g, P); \
+        else                                                                                                     \
+            rc = launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(blocks, st, smem, g, P); \
     } while (0)
+    int rc;
     EK_SUITE_DISPATCH(EK_LAUNCH_SG);
+    if (rc) return rc;
 #undef EK_LAUNCH_SG
     g_launches.fetch_add(1, std::memory_order_relaxed);
     cudaError_t err = cudaGetLastError();

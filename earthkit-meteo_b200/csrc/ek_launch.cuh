@@ -3,6 +3,7 @@
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
+#include <mutex>
 
 #include "../../include/ek_thermo.h"
 #include "ek_thermo_kernels.cuh"
@@ -22,39 +23,59 @@ inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 // Dynamic shared memory of a launch: the lean float64 tables; float32 kernels use none.
 template <typename T> constexpr unsigned smem_for() { return sizeof(T) == 8 ? kSmemBytes : 0u; }
 
-// Once per kernel instantiation and device: ask for a shared-memory carve-out that holds kMinCtas CTAs' tables, so the
-// tables never lower the occupancy the register budget was chosen for (the driver's default carve-out heuristic may
-// pick a smaller one).  `Kernel` is the address of the __global__ instantiation.
-template <auto Kernel> inline void prepare_smem(unsigned smem_bytes) {
-    if (smem_bytes == 0) return;
-    static std::atomic<uint64_t> done{0};
+// Shared-memory attributes of a kernel instantiation on the current device: a carve-out that holds kMinCtas CTAs' worth of
+// `smem_bytes`, so the tables never lower the occupancy the register budget was chosen for (the driver's default carve-out
+// heuristic may pick a smaller one), and, above the 48 KiB default, the dynamic shared memory limit of the function.  `Kernel` is
+// the address of the __global__ instantiation.  The hybrid kernels' size grows with the level count, so the attributes are set
+// again whenever a request exceeds the largest one configured so far on that device; they only ever grow.  Raising them is
+// serialised: with two callers raising at once, the smaller setting must not land after the larger one and break its launches.
+template <auto Kernel> inline int prepare_smem(unsigned smem_bytes) {
+    if (smem_bytes == 0) return EK_OK;
+    constexpr int kDevs = 64;
+    static std::atomic<unsigned> configured[kDevs];  // per device: the largest smem_bytes the attributes hold
+    static std::mutex raising;
     int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0) return;
-    const uint64_t bit = dev < 64 ? (1ull << dev) : 0;
-    if (bit && (done.load(std::memory_order_relaxed) & bit)) return;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0) return EK_OK;  // no current device: the launch reports it
+    std::atomic<unsigned>* have = dev < kDevs ? &configured[dev] : nullptr;
+    if (have && have->load(std::memory_order_acquire) >= smem_bytes) return EK_OK;
+    std::lock_guard<std::mutex> lock(raising);
+    if (have && have->load(std::memory_order_acquire) >= smem_bytes) return EK_OK;
     const unsigned want = kMinCtas * (smem_bytes + 1024u);  // + the per-CTA reservation
     int pct = (int)((want * 100u + 228u * 1024u - 1u) / (228u * 1024u));
     if (pct > 100) pct = 100;
-    cudaFuncSetAttribute(Kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-    if (smem_bytes > 48u * 1024u) cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
-    if (bit) done.fetch_or(bit, std::memory_order_relaxed);
+    cudaFuncSetAttribute(Kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);  // a hint: the launch works without it
+    (void)cudaGetLastError();
+    if (smem_bytes > 48u * 1024u) {
+        const cudaError_t err = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
+        if (err != cudaSuccess) {
+            (void)cudaGetLastError();
+            return set_error((int)err, "cannot allow %u bytes of dynamic shared memory: %s", smem_bytes, cudaGetErrorString(err));
+        }
+    }
+    if (have) {  // max, not store: the value only grows
+        unsigned cur = have->load(std::memory_order_relaxed);
+        while (cur < smem_bytes && !have->compare_exchange_weak(cur, smem_bytes, std::memory_order_release, std::memory_order_relaxed)) {
+        }
+    }
+    return EK_OK;
 }
 
-// prepare_smem + launch of a kernel with the standard CTA size and the dtype's dynamic shared memory
-template <auto Kernel, typename... Args> inline void launch_kernel_smem(int blocks, cudaStream_t st, unsigned smem, Args... args) {
-    prepare_smem<Kernel>(smem);
+// prepare_smem + launch of a kernel with the standard CTA size and the dtype's dynamic shared memory; nonzero: not launched
+template <auto Kernel, typename... Args> inline int launch_kernel_smem(int blocks, cudaStream_t st, unsigned smem, Args... args) {
+    if (int rc = prepare_smem<Kernel>(smem)) return rc;
     Kernel<<<blocks, kThreads, smem, st>>>(args...);
+    return EK_OK;
 }
-template <auto Kernel, typename T, typename... Args> inline void launch_kernel(int blocks, cudaStream_t st, Args... args) {
-    launch_kernel_smem<Kernel>(blocks, st, smem_for<T>(), args...);
+template <auto Kernel, typename T, typename... Args> inline int launch_kernel(int blocks, cudaStream_t st, Args... args) {
+    return launch_kernel_smem<Kernel>(blocks, st, smem_for<T>(), args...);
 }
 
 // Launch of a streaming kernel that orders itself behind its predecessor in the stream with pdl_acquire() (ek_thermo_kernels.cuh):
 // the programmatic-serialization attribute lets it be scheduled while the predecessor drains.  ONLY for kernels that call
 // pdl_acquire() before their first access to a field -- without it the attribute would remove the stream dependency.
 template <auto Kernel, typename... Args>
-inline void launch_streaming(unsigned blocks, unsigned smem, cudaStream_t st, Args... args) {
-    prepare_smem<Kernel>(smem);
+inline int launch_streaming(unsigned blocks, unsigned smem, cudaStream_t st, Args... args) {
+    if (int rc = prepare_smem<Kernel>(smem)) return rc;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(blocks);
     cfg.blockDim = dim3(kThreads);
@@ -66,6 +87,7 @@ inline void launch_streaming(unsigned blocks, unsigned smem, cudaStream_t st, Ar
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     cudaLaunchKernelEx(&cfg, Kernel, args...);
+    return EK_OK;
 }
 
 // Launch Op over n points.  ins[k].ptr == NULL means broadcast scalar ins[k].value; outs[o] == NULL means
@@ -116,7 +138,8 @@ int launch(const char* what, const ek_operand* ins, void* const* outs, int64_t n
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
 
-    launch_streaming<&ew_kernel<Op, OpE, T, unroll>>((unsigned)blocks, smem_for<T>(), static_cast<cudaStream_t>(stream), in, out, n, P, vec_ok);
+    if (int rc = launch_streaming<&ew_kernel<Op, OpE, T, unroll>>((unsigned)blocks, smem_for<T>(), static_cast<cudaStream_t>(stream), in, out, n, P, vec_ok))
+        return rc;
     g_launches.fetch_add(1, std::memory_order_relaxed);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
@@ -180,7 +203,9 @@ int launch_batch(const char* what, int n_seg, const void* const* const* ins, con
         int64_t blocks = ntiles > tail_blocks ? ntiles : tail_blocks;
         if (blocks > cap) blocks = cap;
         if (blocks < 1) blocks = 1;
-        launch_streaming<&ew_batch_kernel<Op, OpE, T, unroll>>((unsigned)blocks, smem_for<T>(), static_cast<cudaStream_t>(stream), B, n_per_seg, P, vec_ok);
+        if (int rc = launch_streaming<&ew_batch_kernel<Op, OpE, T, unroll>>((unsigned)blocks, smem_for<T>(), static_cast<cudaStream_t>(stream), B, n_per_seg, P,
+                                                                            vec_ok))
+            return rc;
         g_launches.fetch_add(1, std::memory_order_relaxed);
         cudaError_t err = cudaGetLastError();
         if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));

@@ -140,12 +140,20 @@ _HM = {"thickness": 0, "geopotential": 1, ("geopotential", "sea"): 2, ("geopoten
 
 
 def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top="ifs", alpha=None, delta=None, zs=None, out=None):
+    """Output form `mode` of the geopotential thickness, one kernel launch.  Computed in the numpy promotion of every array
+    argument; returned in the reference's dtype: the thickness lives in ``zeros_like(R(q) * t)`` (V:806), so its dtype is
+    that of ``t`` / ``q``, and the forms that add ``np.asarray(zs)`` promote it with ``zs`` (a Python number: float64).  A float64
+    computation for float32 ``t`` / ``q`` is rounded once on the way out, as the reference's assignment rounds it.  ``out``, when
+    given, receives the working-dtype result as it is."""
     for x in (t, q):
         if not isinstance(x, torch.Tensor):
             raise TypeError("ek_thermo.vertical: t and q must be torch CUDA tensors (no CPU path)")
     tensors = [x for x in (t, q, sp, alpha, delta, zs) if isinstance(x, torch.Tensor)]
     dev = _b._check_device(tensors)
     dtype = _working_dtype(t, q, sp, alpha, delta, zs, A, B)  # numpy promotion over every array argument, never a down-cast
+    out_dtype = _working_dtype(t, q)
+    if mode in (1, 2, 4, 5):  # the reference adds np.asarray(zs): a Python number is a float64 array there
+        out_dtype = torch.float64 if isinstance(zs, (int, float)) else _working_dtype(t, q, zs)
     if t.shape != q.shape or t.dim() < 1:
         raise ValueError(f"t and q must have the same shape, got {tuple(t.shape)} and {tuple(q.shape)}")
     if vertical_axis != 0:  # V:878-883: work with the vertical axis first
@@ -190,18 +198,22 @@ def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top
         top_toa = _top_is_toa(a, b, nhalf - 1 - nlev, keep[-1], dtype, dev)  # the band is the nlev bottom-most levels (V:1191-1203)
     if mode in (1, 2, 4, 5):
         p_zs = col(zs, "zs")
-    if out is None:
+    own = out is None
+    if own:
         out = torch.empty_like(tc)
     if npl > 0 and nlev > 0:
         _b.call_raw("geopotential_on_hybrid_levels", dtype, dev, c_void_p(tc.data_ptr()), c_void_p(qc.data_ptr()), c_int(nlev), c_int64(npl),
                     p_sp, p_a, p_b, c_int(nhalf), c_int(top_toa), c_double(math.log(2.0) if alpha_top == "ifs" else 1.0), p_al, p_de, p_zs,
                     c_int(mode), c_void_p(out.data_ptr()))
     del keep
+    if own and out.dtype != out_dtype:
+        out = out.to(out_dtype)
     return out.movedim(0, vertical_axis) if vertical_axis != 0 else out
 
 
 def relative_geopotential_thickness_on_hybrid_levels_from_alpha_delta(t, q, alpha, delta, vertical_axis=0):
-    """Geopotential thickness between the surface and the full levels, from precomputed alpha/delta.  Reference V:815-891."""
+    """Geopotential thickness between the surface and the full levels, from precomputed alpha/delta.  Reference V:815-891.
+    Returned in the dtype of ``t`` / ``q`` whatever the dtype of alpha / delta (the reference's ``zeros_like(d)``)."""
     return _column_kernel(t, q, 0, vertical_axis, alpha=alpha, delta=delta)
 
 
@@ -221,8 +233,12 @@ def _thickness_axis_as_reference(t, q, A, B, sp, alpha_top, vertical_axis):
 
 
 def _height_form(dphi, zs, mode):
-    """Output form `mode` of a thickness already in memory, with numpy's broadcasting of zs (and its ValueError)."""
-    zs_t = torch.as_tensor(zs, dtype=None if isinstance(zs, torch.Tensor) else dphi.dtype, device=dphi.device)
+    """Output form `mode` of a thickness already in memory, with numpy's broadcasting of zs (and its ValueError).  Geopotential
+    height above ground does not read zs in the reference (V:1186), so there zs neither broadcasts nor promotes."""
+    if mode == _HM[("geopotential", "ground")]:
+        return _b.execute("height_from_thickness", (dphi, 0.0), (mode,))
+    # np.asarray(zs) in the reference: a Python number is a float64 array, an array keeps its dtype
+    zs_t = torch.as_tensor(zs, dtype=torch.float64 if isinstance(zs, (int, float)) else None, device=dphi.device)
     try:
         torch.broadcast_shapes(tuple(dphi.shape), tuple(zs_t.shape))
     except RuntimeError:
@@ -242,6 +258,10 @@ def geometric_height_from_geopotential(z):
 
 def relative_geopotential_thickness_on_hybrid_levels(t, q, A, B, sp, alpha_top="ifs", vertical_axis=0):
     """Same, with alpha/delta computed inside the kernel from sp and A/B (never materialised).  Reference V:894-994.
+
+    Computed in the numpy promotion of every argument (float64 for Python-list ``A`` / ``B``); returned in the reference's dtype,
+    that of ``t`` / ``q``.  ``geopotential_on_hybrid_levels`` and ``height_on_hybrid_levels`` return that dtype promoted with
+    ``zs`` where they add it (a Python number counts as float64, as ``np.asarray(zs)`` in the reference).
 
     ``t``/``q`` may hold only the bottom-most contiguous levels of the model (V:1191-1203).  ``vertical_axis != 0`` behaves as
     in the reference (see ``_thickness_axis_as_reference``)."""
