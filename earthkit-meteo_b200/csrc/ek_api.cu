@@ -187,7 +187,7 @@ static int host_suite_tq_hybrid(const char* what, const void* h_t, const void* h
     const bool geo = n_col > 0;
     if (geo && h_cols[2] && (height_mode < EK_HM_THICKNESS || height_mode > EK_HM_GEOM_GROUND))
         return set_error(EK_ERR_ENUM, "%s: invalid height mode %d", what, height_mode);
-    const bool zs_row = geo && (h_cols[1] || (h_cols[2] && height_mode != EK_HM_THICKNESS && height_mode != EK_HM_GH_GROUND));
+    const bool zs_row = geo && (h_cols[1] || (h_cols[2] && exactm::height_adds_zs(height_mode)));
     if (zs_row && !h_zs) return set_error(EK_ERR_ARG, "%s: this output needs the surface geopotential zs", what);
     int n_out = 0;
     if (int rc = count_outputs(what, h_outs, out_mask, &n_out, geo)) return rc;

@@ -350,7 +350,7 @@ __global__ void __launch_bounds__(kThreads, (MODE >= EK_HM_GEOM_SEA ? kColMinCta
 #pragma unroll
             for (int j = 0; j < VEC; ++j) phb[j] = exactm::hyb_half(ab, bb, sp[j]);  // V:663
         }
-        const bool add_zs = mode != EK_HM_THICKNESS && mode != EK_HM_GH_GROUND;
+        const bool add_zs = exactm::height_adds_zs(mode);
         if (add_zs) ld_row<T, VECOK>(static_cast<const T*>(g.zs), i0, g.npl, zs, false);
         // The six output forms (V:1064-1069, V:1163-1188) as one expression: z = dphi (+ zs), then nothing / z/g / the
         // geometric height of z minus hsub (geom(zs) or 0: subtracting 0 changes no bit), so the level loop carries
@@ -604,7 +604,7 @@ static int impl_geopotential_on_hybrid_levels(const void* t, const void* q, int 
     if (!t || !q || !out || nlev < 1 || npl < 0 || mode < 0 || mode > 5) return set_error(EK_ERR_ARG, "%s: bad arguments", what);
     if (given && (!alpha || !delta)) return set_error(EK_ERR_ARG, "%s: alpha and delta must be given together", what);
     if (!given && (!sp || !A || !B || nhalf < nlev + 1)) return set_error(EK_ERR_ARG, "%s: sp, A, B (>= nlev + 1 half-levels) are required", what);
-    if ((mode == 1 || mode == 2 || mode == 4 || mode == 5) && !zs) return set_error(EK_ERR_ARG, "%s: this output needs the surface geopotential zs", what);
+    if (exactm::height_adds_zs(mode) && !zs) return set_error(EK_ERR_ARG, "%s: this output needs the surface geopotential zs", what);
     if (npl == 0) return EK_OK;
     GeoArgs g{t, q, sp, A, B, alpha, delta, zs, out, nlev, npl, given ? 0 : nhalf - 1 - nlev, top_toa, alpha_top, mode};
     constexpr int TILE = kThreads * Vec16<T>::N;
@@ -717,7 +717,7 @@ static int suite_hybrid_geo(const void* t, const void* q, const void* sp, const 
     if (!t || !q || !sp || !A || !B || nlev < 1 || npl < 0) return set_error(EK_ERR_ARG, "%s: bad arguments", what);
     if (height_out && (height_mode < EK_HM_THICKNESS || height_mode > EK_HM_GEOM_GROUND))
         return set_error(EK_ERR_ENUM, "%s: invalid height mode %d", what, height_mode);
-    const bool need_zs = z_out || (height_out && height_mode != EK_HM_THICKNESS && height_mode != EK_HM_GH_GROUND);
+    const bool need_zs = z_out || (height_out && exactm::height_adds_zs(height_mode));
     if (need_zs && !zs) return set_error(EK_ERR_ARG, "%s: this output needs the surface geopotential zs", what);
     SuiteGeoArgs g{t, q, sp, need_zs ? zs : nullptr, A, B, {}, p_out, thickness_out, z_out, height_out, nlev, npl, top_toa, alpha_top,
                    height_out ? height_mode : EK_HM_THICKNESS};

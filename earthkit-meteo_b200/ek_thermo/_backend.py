@@ -9,6 +9,7 @@ import ctypes
 import os
 from ctypes import c_double, c_int, c_int64, c_size_t, c_uint32, c_uint64, c_void_p
 
+import numpy as np
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -39,6 +40,9 @@ _lib.ek_thermo_set_launch_config.argtypes = [c_int, c_int]
 _lib.ek_thermo_shard_range.argtypes = [c_int64, c_int, c_int, c_int64, ctypes.POINTER(c_int64), ctypes.POINTER(c_int64)]
 
 _SUFFIX = {torch.float64: "f64", torch.float32: "f32"}
+_TORCH = {np.dtype("float64"): torch.float64, np.dtype("float32"): torch.float32}  # the host-array dtypes and their tensor dtypes
+# ept_method -> EK_EPT_* (T:1319-1323); an unknown method is a KeyError, as in the reference (T:1024-1026)
+_EPT = {"ifs": 0, "bolton35": 1, "bolton39": 2}
 
 # option kinds of every entry point, in C argument order:  operands..., options..., outputs..., n, stream
 # name -> (n_inputs, option ctypes, n_outputs)
@@ -411,12 +415,10 @@ def execute_suite_batch(symbol: str, seg_args, out_names, slots, outs=None, ept_
             for t in a:
                 if t.dtype != dtype or t.shape != shape or not t.is_contiguous():
                     raise ValueError("ek_thermo: the fields of a batched suite must share dtype, device and shape and be contiguous")
-            arr = (c_void_p * n_seg)(*[t.data_ptr() for t in a])
-            keep.append(arr)
-            ptr_arrays.append(ctypes.cast(arr, c_void_p))
+            ptr_arrays.append((c_void_p * n_seg)(*[t.data_ptr() for t in a]))
         elif isinstance(a, (int, float)) and not isinstance(a, bool):
             scalars[k] = float(a)
-            ptr_arrays.append(c_void_p(None))
+            ptr_arrays.append(None)
         else:
             raise TypeError("ek_thermo: batched suite arguments are lists of CUDA tensors or Python numbers")
     out_tab = (c_void_p * N_SUITE_SLOTS)()
@@ -450,35 +452,10 @@ def shard_range(n: int, world: int, rank: int, align: int = 1):
     return int(b.value), int(e.value)
 
 
-def host_suite(kind: int, dtype, h_ptrs, h_out_ptrs, mask: int, ept_method: int, n: int, workspace: torch.Tensor, n_slots: int):
-    fn = getattr(_lib, f"ek_thermo_host_suite_{_SUFFIX[dtype]}")
-    outs = (c_void_p * N_SUITE_SLOTS)(*h_out_ptrs)
+def host_pipeline(symbol: str, dtype, workspace: torch.Tensor, n_slots: int, *c_args):
+    """Run host-array pipeline entry point `symbol` (ek_thermo_host_suite*): `c_args` up to the workspace, which the pipeline
+    splits into `n_slots` stream slots."""
+    fn = getattr(_lib, f"ek_thermo_{symbol}_{_SUFFIX[dtype]}")
     with torch.cuda.device(workspace.device):
         torch.cuda.current_stream().synchronize()  # the pipeline runs on its own streams: nothing may be pending on the workspace
-        _check(fn(kind, c_void_p(h_ptrs[0]), c_void_p(h_ptrs[1]), c_void_p(h_ptrs[2]), ctypes.cast(outs, ctypes.POINTER(c_void_p)),
-                  c_uint32(mask), c_int(ept_method), c_int64(n), c_void_p(workspace.data_ptr()),
-                  c_size_t(workspace.numel() * workspace.element_size()), c_int(n_slots)))
-
-
-def host_suite_tq_hybrid(dtype, h_t, h_q, h_sp, h_a, h_b, nlev: int, npl: int, h_out_ptrs, mask: int, ept_method: int, workspace: torch.Tensor,
-                         n_slots: int):
-    fn = getattr(_lib, f"ek_thermo_host_suite_tq_hybrid_{_SUFFIX[dtype]}")
-    outs = (c_void_p * N_SUITE_SLOTS)(*h_out_ptrs)
-    with torch.cuda.device(workspace.device):
-        torch.cuda.current_stream().synchronize()
-        _check(fn(c_void_p(h_t), c_void_p(h_q), c_void_p(h_sp), c_void_p(h_a), c_void_p(h_b), c_int(nlev), c_int64(npl),
-                  ctypes.cast(outs, ctypes.POINTER(c_void_p)), c_uint32(mask), c_int(ept_method), c_void_p(workspace.data_ptr()),
-                  c_size_t(workspace.numel() * workspace.element_size()), c_int(n_slots)))
-
-
-def host_suite_tq_hybrid_geo(dtype, h_t, h_q, h_sp, h_zs, h_a, h_b, nlev: int, npl: int, h_out_ptrs, mask: int, ept_method: int, top_toa: int,
-                             alpha_top: float, h_cols, height_mode: int, workspace: torch.Tensor, n_slots: int):
-    """``h_cols``: host pointers (or None) of the thickness, z and height outputs."""
-    fn = getattr(_lib, f"ek_thermo_host_suite_tq_hybrid_geo_{_SUFFIX[dtype]}")
-    outs = (c_void_p * N_SUITE_SLOTS)(*h_out_ptrs)
-    with torch.cuda.device(workspace.device):
-        torch.cuda.current_stream().synchronize()
-        _check(fn(c_void_p(h_t), c_void_p(h_q), c_void_p(h_sp), c_void_p(h_zs), c_void_p(h_a), c_void_p(h_b), c_int(nlev), c_int64(npl),
-                  ctypes.cast(outs, ctypes.POINTER(c_void_p)), c_uint32(mask), c_int(ept_method), c_int(top_toa), c_double(alpha_top),
-                  *(c_void_p(p) for p in h_cols), c_int(height_mode), c_void_p(workspace.data_ptr()),
-                  c_size_t(workspace.numel() * workspace.element_size()), c_int(n_slots)))
+        _check(fn(*c_args, workspace.data_ptr(), workspace.numel() * workspace.element_size(), n_slots))

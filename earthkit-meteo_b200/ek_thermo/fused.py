@@ -7,9 +7,14 @@ named in ``SUITE_TQP_OUTPUTS`` / ``SUITE_TTDP_OUTPUTS`` applied to the same inpu
 """
 from __future__ import annotations
 
-import math
+from ctypes import c_void_p
+
+import torch
 
 from . import _backend as _b
+from ._backend import _EPT
+from .vertical import COLUMN_OUTPUTS  # noqa: F401  (part of this module's API: the column outputs of suite_tq_hybrid)
+from .vertical import _alpha_top_value, _column_kernel, _split_suite_outputs, _top_is_toa
 
 # output name -> slot (include/ek_thermo.h EK_S_*), with the reference function each one equals
 SUITE_TQP_OUTPUTS = {
@@ -45,7 +50,6 @@ ALL7_TTDP = ("theta", "es", "rh", "q", "tv", "ept", "wbpt")
 DEFAULT_TQP = ("theta", "es", "rh", "td", "tv")
 DEFAULT_TTDP = ("theta", "es", "rh", "q", "tv")
 
-_EPT = {"ifs": 0, "bolton35": 1, "bolton39": 2}
 _TM = {None: 0, "none": 0, "direct": 1, "bisect": 2, "newton": 3}
 
 
@@ -57,7 +61,7 @@ def _slots(table, outputs):
 
 
 def _ept_id(ept_method):
-    return _EPT[ept_method]  # KeyError for an unknown method, as the reference (T:1026)
+    return _EPT[ept_method]
 
 
 def suite_tqp(t, q, p, outputs=DEFAULT_TQP, out=None, ept_method="ifs"):
@@ -92,12 +96,6 @@ def suite_ttdp_batch(ts, tds, ps, outputs=DEFAULT_TTDP, out=None, ept_method="if
     return _b.execute_suite_batch("suite_ttdp_batch", (ts, tds, ps), outputs, _slots(SUITE_TTDP_OUTPUTS, outputs), out, _ept_id(ept_method))
 
 
-# column outputs of suite_tq_hybrid: the geopotential of the same levels, from the same walk of the columns
-COLUMN_OUTPUTS = (
-    "thickness",  # relative_geopotential_thickness_on_hybrid_levels(t, q, A, B, sp, alpha_top)                      V:894-994
-    "z",  # geopotential_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top)                                            V:997-1069
-    "height",  # height_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top, h_type, h_reference)                        V:1072-1188
-)
 # Fields of fewer columns than this run a mixed call as the suite launch plus one geopotential_on_hybrid_levels launch per column
 # output: the fused walk has one work item per tile of 256 threads x one 16-byte vector of columns (512 columns in float64, 1024 in
 # float32), so a small field leaves most of the GPU idle, while the suite launch also splits the levels into work items.  Measured
@@ -108,8 +106,6 @@ GEO_FUSED_MIN_COLUMNS = {"float64": 65536, "float32": 262144}
 
 def _out_buffer(out, name, like):
     """out[name] when the caller preallocated it (checked), else a new tensor like `like`."""
-    import torch
-
     if out is not None and name in out:
         o = out[name]
         if o.dtype != like.dtype or o.shape != like.shape or not o.is_contiguous() or o.device != like.device:
@@ -138,20 +134,10 @@ def suite_tq_hybrid(t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, want_p=False,
     the ``ek_thermo.vertical`` functions called with ``A`` / ``B`` given as tensors of that dtype (not the float64 promotion
     those functions apply to Python-list ``A`` / ``B``).
     """
-    import ctypes
-    from ctypes import c_double, c_int, c_int64, c_uint32, c_void_p
-
-    import torch
-
-    from .vertical import _column_kernel, _height_mode, _top_is_toa
-
     outputs = tuple(outputs)
-    cols = tuple(o for o in outputs if o in COLUMN_OUTPUTS)
-    suite = tuple(o for o in outputs if o not in COLUMN_OUTPUTS)
+    alpha_top_value = _alpha_top_value(alpha_top)
+    suite, cols, need_zs = _split_suite_outputs(outputs, h_type, h_reference, zs)
     slots = _slots(SUITE_TQP_OUTPUTS, suite)
-    if alpha_top not in ("ifs", "arpege"):
-        raise ValueError(f"Unknown method '{alpha_top}' for pressure calculation. Use 'ifs' or 'arpege'.")
-    hmode = _height_mode(h_type, h_reference)
     for x in (t, q, sp):
         if not isinstance(x, torch.Tensor):
             raise TypeError("suite_tq_hybrid: t, q and sp must be torch CUDA tensors")
@@ -166,10 +152,7 @@ def suite_tq_hybrid(t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, want_p=False,
     b = torch.as_tensor(B, dtype=dtype, device=dev).contiguous()
     if a.numel() != nlev + 1 or b.numel() != nlev + 1:
         raise ValueError(f"suite_tq_hybrid: A and B need nlev + 1 = {nlev + 1} half-level values")
-    modes = {"thickness": 0, "z": 1, "height": hmode}
-    if any(modes[c] not in (0, 3) for c in cols):
-        if zs is None:
-            raise ValueError("suite_tq_hybrid: 'z' and every 'height' except geopotential height above ground need the surface geopotential zs")
+    if need_zs:
         if isinstance(zs, torch.Tensor):
             _b._check_device([t, zs])
             if zs.dtype != dtype or zs.shape != sp.shape:
@@ -188,29 +171,27 @@ def suite_tq_hybrid(t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, want_p=False,
     for name, k in zip(suite, slots):
         ptrs[k] = res[name].data_ptr()
         mask |= 1 << k
-    p_ptr = c_void_p(None)
+    p_ptr = None
     if want_p:
         res["p"] = _out_buffer(out, "p", tc)
-        p_ptr = c_void_p(res["p"].data_ptr())
+        p_ptr = res["p"].data_ptr()
     if npl == 0:
         return res
     fused = bool(cols) and (bool(suite) or want_p) and npl >= GEO_FUSED_MIN_COLUMNS["float64" if dtype == torch.float64 else "float32"]
     if not fused and (suite or want_p or not cols):
-        _b.call_raw("suite_tq_hybrid", dtype, dev, c_void_p(tc.data_ptr()), c_void_p(qc.data_ptr()), c_void_p(spc.data_ptr()),
-                    c_void_p(a.data_ptr()), c_void_p(b.data_ptr()), c_int(nlev), c_int64(npl), ctypes.cast(ptrs, ctypes.POINTER(c_void_p)),
-                    c_uint32(mask), c_int(em), p_ptr)
+        _b.call_raw("suite_tq_hybrid", dtype, dev, tc.data_ptr(), qc.data_ptr(), spc.data_ptr(), a.data_ptr(), b.data_ptr(), nlev, npl, ptrs, mask,
+                    em, p_ptr)
     if not fused:
-        for name in cols:
-            _column_kernel(tc, qc, modes[name], 0, sp=spc, A=a, B=b, alpha_top=alpha_top, zs=zs, out=res[name])
+        for name, mode in cols.items():
+            _column_kernel(tc, qc, mode, 0, sp=spc, A=a, B=b, alpha_top=alpha_top, zs=zs, out=res[name])
         return res
     zsc = None
     if zs is not None:
         zsc = zs.contiguous() if isinstance(zs, torch.Tensor) else torch.full(tuple(sp.shape), float(zs), dtype=dtype, device=dev)
-    col_ptr = lambda n: c_void_p(res[n].data_ptr()) if n in res else c_void_p(None)  # noqa: E731
-    _b.call_raw("suite_tq_hybrid_geo", dtype, dev, c_void_p(tc.data_ptr()), c_void_p(qc.data_ptr()), c_void_p(spc.data_ptr()),
-                c_void_p(zsc.data_ptr() if zsc is not None else None), c_void_p(a.data_ptr()), c_void_p(b.data_ptr()), c_int(nlev), c_int64(npl),
-                ctypes.cast(ptrs, ctypes.POINTER(c_void_p)), c_uint32(mask), c_int(em), p_ptr, c_int(_top_is_toa(a, b, 0, spc, dtype, dev)),
-                c_double(math.log(2.0) if alpha_top == "ifs" else 1.0), col_ptr("thickness"), col_ptr("z"), col_ptr("height"), c_int(hmode))
+    col_ptr = lambda n: res[n].data_ptr() if n in res else None  # noqa: E731
+    _b.call_raw("suite_tq_hybrid_geo", dtype, dev, tc.data_ptr(), qc.data_ptr(), spc.data_ptr(), zsc.data_ptr() if zsc is not None else None,
+                a.data_ptr(), b.data_ptr(), nlev, npl, ptrs, mask, em, p_ptr, _top_is_toa(a, b, 0, spc, dtype, dev), alpha_top_value,
+                col_ptr("thickness"), col_ptr("z"), col_ptr("height"), cols.get("height", 0))
     return res
 
 

@@ -28,11 +28,11 @@ import torch
 from . import fused as _fused
 from . import thermo as _thermo
 from . import wind as _wind
+from ._backend import _TORCH
 
 __all__ = ["thermo", "wind", "fused", "set_chunk_elements", "set_pinned_results", "release_staging"]
 
 _CHUNK = 1 << 25  # elements per array per chunk (256 MB of float64): bounds device memory, amortises launch latency
-_TORCH = {np.dtype("float64"): torch.float64, np.dtype("float32"): torch.float32}
 
 
 def set_chunk_elements(n):

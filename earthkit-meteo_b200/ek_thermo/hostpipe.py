@@ -6,15 +6,15 @@ several streams (ek_thermo_host_suite_*).  All arithmetic still happens on the G
 """
 from __future__ import annotations
 
-import math
+from ctypes import c_void_p
 
 import numpy as np
 import torch
 
 from . import _backend as _b
-from .fused import COLUMN_OUTPUTS, DEFAULT_TQP, DEFAULT_TTDP, SUITE_TQP_OUTPUTS, SUITE_TTDP_OUTPUTS
-
-_TORCH = {np.dtype("float64"): torch.float64, np.dtype("float32"): torch.float32}
+from ._backend import _EPT, _TORCH
+from .fused import DEFAULT_TQP, DEFAULT_TTDP, SUITE_TQP_OUTPUTS, SUITE_TTDP_OUTPUTS
+from .vertical import COLUMN_OUTPUTS, _alpha_top_value, _split_suite_outputs, _top_is_toa
 
 
 def pinned_empty(n, dtype=np.float64):
@@ -58,9 +58,6 @@ def bind_host_to_device(device="cuda:0"):
         return None
 
 
-_EPT = {"ifs": 0, "bolton35": 1, "bolton39": 2}
-
-
 class HostSuite:
     """Reusable pipeline: owns the device workspace (allocated once through torch) and the stream slots."""
 
@@ -72,7 +69,7 @@ class HostSuite:
     @staticmethod
     def _outputs(table, outputs, out, shape, dt):
         n = int(np.prod(shape))
-        ptrs = [0] * _b.N_SUITE_SLOTS
+        ptrs = (c_void_p * _b.N_SUITE_SLOTS)()
         mask = 0
         res = {}
         for name in outputs:
@@ -91,7 +88,8 @@ class HostSuite:
         if dt not in _TORCH or any(x.dtype != dt or x.shape != arrs[0].shape for x in arrs):
             raise TypeError("host suite: the three inputs must be float64 or float32 numpy arrays of one shape")
         res, ptrs, mask = self._outputs(table, outputs, out, arrs[0].shape, dt)
-        _b.host_suite(kind, _TORCH[dt], [x.ctypes.data for x in arrs], ptrs, mask, _EPT[ept_method], arrs[0].size, self.workspace, self.n_slots)
+        _b.host_pipeline("host_suite", _TORCH[dt], self.workspace, self.n_slots, kind, *(x.ctypes.data for x in arrs), ptrs, mask, _EPT[ept_method],
+                         arrs[0].size)
         return res
 
     def suite_tqp(self, t, q, p, outputs=DEFAULT_TQP, out=None, ept_method="ifs"):
@@ -106,14 +104,9 @@ class HostSuite:
         The pressure field crosses PCIe in neither direction (sp travels instead: 16 + 8/nlev bytes per point in).  The column
         outputs ``"thickness"``, ``"z"`` and ``"height"`` with ``zs`` (a ``[npl]`` array or a Python number), ``alpha_top``,
         ``h_type`` and ``h_reference`` as there; they come from the same kernel pass over each chunk."""
-        from .vertical import _height_mode, _top_is_toa
-
         outputs = tuple(outputs)
-        cols = tuple(o for o in outputs if o in COLUMN_OUTPUTS)
-        suite = tuple(o for o in outputs if o not in COLUMN_OUTPUTS)
-        if alpha_top not in ("ifs", "arpege"):
-            raise ValueError(f"Unknown method '{alpha_top}' for pressure calculation. Use 'ifs' or 'arpege'.")
-        hmode = _height_mode(h_type, h_reference)
+        alpha_top_value = _alpha_top_value(alpha_top)
+        suite, cols, need_zs = _split_suite_outputs(outputs, h_type, h_reference, zs)
         t, q, sp = (np.ascontiguousarray(x) for x in (t, q, sp))
         dt = t.dtype
         if dt not in _TORCH or q.dtype != dt or sp.dtype != dt or t.ndim != 2 or q.shape != t.shape or sp.shape != t.shape[1:]:
@@ -125,14 +118,11 @@ class HostSuite:
             raise ValueError(f"host suite: A and B need nlev + 1 = {nlev + 1} half-level values")
         res, ptrs, mask = self._outputs(SUITE_TQP_OUTPUTS, suite, out, t.shape, dt)
         if not cols:
-            _b.host_suite_tq_hybrid(_TORCH[dt], t.ctypes.data, q.ctypes.data, sp.ctypes.data, a.ctypes.data, b.ctypes.data, nlev, npl, ptrs, mask,
-                                    _EPT[ept_method], self.workspace, self.n_slots)
+            _b.host_pipeline("host_suite_tq_hybrid", _TORCH[dt], self.workspace, self.n_slots, t.ctypes.data, q.ctypes.data, sp.ctypes.data,
+                             a.ctypes.data, b.ctypes.data, nlev, npl, ptrs, mask, _EPT[ept_method])
             return res
-        modes = {"thickness": 0, "z": 1, "height": hmode}
         zs_ptr = None
-        if any(modes[c] not in (0, 3) for c in cols):
-            if zs is None:
-                raise ValueError("host suite: 'z' and every 'height' except geopotential height above ground need the surface geopotential zs")
+        if need_zs:
             zs = np.full(sp.shape, zs, dtype=dt) if isinstance(zs, (int, float)) and not isinstance(zs, bool) else np.ascontiguousarray(zs)
             if zs.dtype != dt or zs.shape != sp.shape:
                 raise TypeError(f"host suite: zs must be a {dt} array of shape {sp.shape} or a Python number")
@@ -140,7 +130,7 @@ class HostSuite:
         col_res, _, _ = self._outputs({c: 0 for c in cols}, cols, out, t.shape, dt)
         res.update(col_res)
         res = {name: res[name] for name in outputs}
-        _b.host_suite_tq_hybrid_geo(_TORCH[dt], t.ctypes.data, q.ctypes.data, sp.ctypes.data, zs_ptr, a.ctypes.data, b.ctypes.data, nlev, npl, ptrs,
-                                    mask, _EPT[ept_method], _top_is_toa(a, b, 0, sp, None, None), math.log(2.0) if alpha_top == "ifs" else 1.0,
-                                    [res[c].ctypes.data if c in res else None for c in COLUMN_OUTPUTS], hmode, self.workspace, self.n_slots)
+        _b.host_pipeline("host_suite_tq_hybrid_geo", _TORCH[dt], self.workspace, self.n_slots, t.ctypes.data, q.ctypes.data, sp.ctypes.data, zs_ptr,
+                         a.ctypes.data, b.ctypes.data, nlev, npl, ptrs, mask, _EPT[ept_method], _top_is_toa(a, b, 0, sp, None, None), alpha_top_value,
+                         *(res[c].ctypes.data if c in res else None for c in COLUMN_OUTPUTS), cols.get("height", 0))
         return res

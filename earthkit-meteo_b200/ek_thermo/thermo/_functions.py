@@ -13,10 +13,10 @@ N-D, SURVEY.md §7.3-H6).
 from __future__ import annotations
 
 from .. import _backend as _b
+from .._backend import _EPT
 
 _PHASE = {"mixed": 0, "water": 1, "ice": 2}  # E:22
 _LCL = {"davies": 0, "bolton": 1}  # T:960-968
-_EPT = {"ifs": 0, "bolton35": 1, "bolton39": 2}  # T:1319-1323
 _TM = {"direct": 1, "bisect": 2, "newton": 3}
 
 __all__ = [

@@ -7,7 +7,6 @@ One kernel launch reads ``sp`` once and writes every requested [level, point] ar
 from __future__ import annotations
 
 import math
-from ctypes import c_double, c_int, c_int64, c_void_p
 
 import numpy as np
 import torch
@@ -66,9 +65,15 @@ def _top_is_toa(a, b, top_half, spc, dtype, dev):
     if host:
         return int(np.any(a[top_half] + b[top_half] * spc <= spc.dtype.type(0.1)))
     flag = torch.zeros(1, dtype=torch.int32, device=dev)
-    _b.call_raw("hybrid_top_is_toa", dtype, dev, c_void_p(spc.data_ptr()), c_int64(spc.numel()), c_double(a_top), c_double(b_top),
-                c_void_p(flag.data_ptr()))
+    _b.call_raw("hybrid_top_is_toa", dtype, dev, spc.data_ptr(), spc.numel(), a_top, b_top, flag.data_ptr())
     return int(flag.item())
+
+
+def _alpha_top_value(alpha_top):
+    """alpha of the top level when its upper half level is the top of the atmosphere: ln 2 for "ifs", 1 for "arpege" (V:669)."""
+    if alpha_top not in ("ifs", "arpege"):
+        raise ValueError(f"Unknown method '{alpha_top}' for pressure calculation. Use 'ifs' or 'arpege'.")  # V:626-627
+    return math.log(2.0) if alpha_top == "ifs" else 1.0
 
 
 def pressure_on_hybrid_levels(A, B, sp, levels=None, alpha_top="ifs", output="full", vertical_axis=0):
@@ -86,8 +91,7 @@ def pressure_on_hybrid_levels(A, B, sp, levels=None, alpha_top="ifs", output="fu
     for out in output:
         if out not in _OUTPUTS:
             raise ValueError(f"Unknown output type '{out}'. Allowed values are 'full', 'half', 'alpha' or 'delta'.")  # V:620-624
-    if alpha_top not in ("ifs", "arpege"):
-        raise ValueError(f"Unknown method '{alpha_top}' for pressure calculation. Use 'ifs' or 'arpege'.")  # V:626-627
+    alpha_top_value = _alpha_top_value(alpha_top)
     if not isinstance(sp, torch.Tensor):
         raise TypeError("ek_thermo.vertical: sp must be a torch CUDA tensor (no CPU path; use earthkit.meteo.vertical for host arrays)")
     dev = _b._check_device([sp])
@@ -120,12 +124,11 @@ def pressure_on_hybrid_levels(A, B, sp, levels=None, alpha_top="ifs", output="fu
             # alpha / delta: xp.zeros(...) arrays in the reference, i.e. always float64 (V:672,686); the kernel widens on store
             odt = torch.float64 if name in ("alpha", "delta") else dtype
             res[name] = torch.empty((nrow,) + tuple(sp.shape), dtype=odt, device=dev)
-    ptr = lambda n: c_void_p(res[n].data_ptr()) if n in res else c_void_p(None)  # noqa: E731
+    ptr = lambda n: res[n].data_ptr() if n in res else None  # noqa: E731
     if npl > 0:
-        _b.call_raw("pressure_on_hybrid_levels", dtype, dev, c_void_p(a.data_ptr()), c_void_p(b.data_ptr()), c_int(nhalf),
-                    c_void_p(spc.data_ptr()), c_int64(npl), c_void_p(rows_f.data_ptr()), c_int(len(full_rows)), c_void_p(rows_h.data_ptr()),
-                    c_int(len(half_rows)), c_int(top_k), c_int(top_toa), c_double(math.log(2.0) if alpha_top == "ifs" else 1.0),
-                    ptr("full"), ptr("half"), ptr("delta"), ptr("alpha"), c_int(1))
+        _b.call_raw("pressure_on_hybrid_levels", dtype, dev, a.data_ptr(), b.data_ptr(), nhalf, spc.data_ptr(), npl, rows_f.data_ptr(),
+                    len(full_rows), rows_h.data_ptr(), len(half_rows), top_k, top_toa, alpha_top_value, ptr("full"), ptr("half"), ptr("delta"),
+                    ptr("alpha"), 1)
     outs = [res[o] for o in output]
     if vertical_axis != 0 and outs[0].dim() > 1:  # V:731-733
         outs = [r.movedim(0, vertical_axis) for r in outs]
@@ -137,6 +140,11 @@ def pressure_on_hybrid_levels(A, B, sp, levels=None, alpha_top="ifs", output="fu
 # --------------------------------------------------------------------------------------------------------------------
 _HM = {"thickness": 0, "geopotential": 1, ("geopotential", "sea"): 2, ("geopotential", "ground"): 3, ("geometric", "sea"): 4,
        ("geometric", "ground"): 5}
+
+
+def _adds_zs(mode):
+    """Does height form `mode` add the surface geopotential zs?  All but the thickness and geopotential height above ground (V:1186)."""
+    return mode != _HM["thickness"] and mode != _HM[("geopotential", "ground")]
 
 
 def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top="ifs", alpha=None, delta=None, zs=None, out=None):
@@ -152,7 +160,7 @@ def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top
     dev = _b._check_device(tensors)
     dtype = _working_dtype(t, q, sp, alpha, delta, zs, A, B)  # numpy promotion over every array argument, never a down-cast
     out_dtype = _working_dtype(t, q)
-    if mode in (1, 2, 4, 5):  # the reference adds np.asarray(zs): a Python number is a float64 array there
+    if _adds_zs(mode):  # the reference adds np.asarray(zs): a Python number is a float64 array there
         out_dtype = torch.float64 if isinstance(zs, (int, float)) else _working_dtype(t, q, zs)
     if t.shape != q.shape or t.dim() < 1:
         raise ValueError(f"t and q must have the same shape, got {tuple(t.shape)} and {tuple(q.shape)}")
@@ -164,7 +172,6 @@ def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top
     nlev = int(tc.shape[0])
     col_shape = tuple(tc.shape[1:])
     npl = int(tc[0].numel()) if nlev else 0
-    null = c_void_p(None)
     keep = []
 
     def col(x, name):  # a per-column field (sp, zs): broadcast to the column shape
@@ -173,10 +180,11 @@ def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top
             x = x.expand(col_shape)
         x = x.contiguous()
         keep.append(x)
-        return c_void_p(x.data_ptr())
+        return x.data_ptr()
 
-    p_sp = p_a = p_b = p_al = p_de = p_zs = null
+    p_sp = p_a = p_b = p_al = p_de = p_zs = None
     nhalf = top_toa = 0
+    alpha_top_value = _alpha_top_value(alpha_top)
     if alpha is not None:
         if alpha.shape != t.shape or delta.shape != t.shape:  # numpy broadcasting of d * alpha, d * delta into zeros_like(d) (V:804-810)
             try:
@@ -185,26 +193,23 @@ def _column_kernel(t, q, mode, vertical_axis, sp=None, A=None, B=None, alpha_top
                 raise ValueError(f"operands could not be broadcast together with shapes {tuple(t.shape)} {tuple(alpha.shape)}") from None
         ac, dc = alpha.to(dtype).contiguous(), delta.to(dtype).contiguous()
         keep += [ac, dc]
-        p_al, p_de = c_void_p(ac.data_ptr()), c_void_p(dc.data_ptr())
+        p_al, p_de = ac.data_ptr(), dc.data_ptr()
     else:
-        if alpha_top not in ("ifs", "arpege"):
-            raise ValueError(f"Unknown method '{alpha_top}' for pressure calculation. Use 'ifs' or 'arpege'.")
         a, b = _coeff_tensors(A, B, dtype, dev)
         nhalf = a.numel()
         if nlev > nhalf - 1:
             raise ValueError(f"Requested level {nlev} exceeds the maximum number of levels {nhalf - 1}.")
         keep += [a, b]
-        p_a, p_b, p_sp = c_void_p(a.data_ptr()), c_void_p(b.data_ptr()), col(sp, "sp")
+        p_a, p_b, p_sp = a.data_ptr(), b.data_ptr(), col(sp, "sp")
         top_toa = _top_is_toa(a, b, nhalf - 1 - nlev, keep[-1], dtype, dev)  # the band is the nlev bottom-most levels (V:1191-1203)
-    if mode in (1, 2, 4, 5):
+    if _adds_zs(mode):
         p_zs = col(zs, "zs")
     own = out is None
     if own:
         out = torch.empty_like(tc)
     if npl > 0 and nlev > 0:
-        _b.call_raw("geopotential_on_hybrid_levels", dtype, dev, c_void_p(tc.data_ptr()), c_void_p(qc.data_ptr()), c_int(nlev), c_int64(npl),
-                    p_sp, p_a, p_b, c_int(nhalf), c_int(top_toa), c_double(math.log(2.0) if alpha_top == "ifs" else 1.0), p_al, p_de, p_zs,
-                    c_int(mode), c_void_p(out.data_ptr()))
+        _b.call_raw("geopotential_on_hybrid_levels", dtype, dev, tc.data_ptr(), qc.data_ptr(), nlev, npl, p_sp, p_a, p_b, nhalf, top_toa,
+                    alpha_top_value, p_al, p_de, p_zs, mode, out.data_ptr())
     del keep
     if own and out.dtype != out_dtype:
         out = out.to(out_dtype)
@@ -235,7 +240,7 @@ def _thickness_axis_as_reference(t, q, A, B, sp, alpha_top, vertical_axis):
 def _height_form(dphi, zs, mode):
     """Output form `mode` of a thickness already in memory, with numpy's broadcasting of zs (and its ValueError).  Geopotential
     height above ground does not read zs in the reference (V:1186), so there zs neither broadcasts nor promotes."""
-    if mode == _HM[("geopotential", "ground")]:
+    if not _adds_zs(mode):
         return _b.execute("height_from_thickness", (dphi, 0.0), (mode,))
     # np.asarray(zs) in the reference: a Python number is a float64 array, an array keeps its dtype
     zs_t = torch.as_tensor(zs, dtype=torch.float64 if isinstance(zs, (int, float)) else None, device=dphi.device)
@@ -282,6 +287,27 @@ def _height_mode(h_type, h_reference):
     if h_reference not in ["sea", "ground"]:
         raise ValueError(f"Unknown '{h_reference=}'. Use 'sea' or 'ground'.")  # V:1163-1164
     return _HM[("geometric" if h_type == "geometric" else "geopotential", h_reference)]  # any other h_type -> geopotential (V:1175-1186)
+
+
+# column outputs of fused.suite_tq_hybrid and hostpipe.HostSuite.suite_tq_hybrid: the geopotential of the suite's levels, from the
+# same walk of the columns
+COLUMN_OUTPUTS = (
+    "thickness",  # relative_geopotential_thickness_on_hybrid_levels(t, q, A, B, sp, alpha_top)                      V:894-994
+    "z",  # geopotential_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top)                                            V:997-1069
+    "height",  # height_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top, h_type, h_reference)                        V:1072-1188
+)
+
+
+def _split_suite_outputs(outputs, h_type, h_reference, zs):
+    """``outputs`` of a hybrid-level suite call as (suite outputs, {column output: height mode}, whether zs is read).  Raises
+    ValueError when a column output needs zs and none is given."""
+    modes = dict(zip(COLUMN_OUTPUTS, (_HM["thickness"], _HM["geopotential"], _height_mode(h_type, h_reference))))
+    suite = tuple(o for o in outputs if o not in modes)
+    cols = {o: modes[o] for o in outputs if o in modes}
+    need_zs = any(_adds_zs(m) for m in cols.values())
+    if need_zs and zs is None:
+        raise ValueError("suite_tq_hybrid: 'z' and every 'height' except geopotential height above ground need the surface geopotential zs")
+    return suite, cols, need_zs
 
 
 def height_on_hybrid_levels(t, q, zs, A, B, sp, alpha_top="ifs", h_type="geometric", h_reference="ground", vertical_axis=0):

@@ -73,7 +73,7 @@ def test_host_suite_argument_errors(monkeypatch):
     import ek_thermo
     from ek_thermo import hostpipe
 
-    monkeypatch.setattr(ek_thermo._backend, "host_suite_tq_hybrid_geo", lambda *a, **k: pytest.fail("the pipeline was entered"))
+    monkeypatch.setattr(ek_thermo._backend, "host_pipeline", lambda *a, **k: pytest.fail("the pipeline was entered"))
     hs = object.__new__(hostpipe.HostSuite)  # no device workspace needed for the checks
     t = np.ones((3, 5))
     sp = np.full(5, 1.0e5)
