@@ -105,17 +105,6 @@ struct StreamSet {
         return EK_OK;
     }
 };
-
-int count_outputs(const char* what, void* const* h_outs, uint32_t out_mask, int* n_out, bool allow_none = false) {
-    if ((out_mask == 0 && !allow_none) || out_mask >= (1u << S_NSLOTS)) return set_error(EK_ERR_ARG, "%s: out_mask=0x%x", what, out_mask);
-    *n_out = 0;
-    for (int k = 0; k < S_NSLOTS; ++k)
-        if ((out_mask >> k) & 1u) {
-            if (!h_outs[k]) return set_error(EK_ERR_ARG, "%s: output %d requested but its buffer is NULL", what, k);
-            ++*n_out;
-        }
-    return EK_OK;
-}
 }  // namespace
 
 template <typename T>
@@ -124,11 +113,11 @@ static int impl_host_suite(int kind, const void* h_a, const void* h_b, const voi
     if (kind != 0 && kind != 1) return set_error(EK_ERR_ENUM, "host_suite: kind=%d", kind);
     if (!h_a || !h_b || !h_c || !h_outs || !workspace) return set_error(EK_ERR_ARG, "host_suite: NULL buffer");
     if (n < 0 || n_slots < 1 || n_slots > 16) return set_error(EK_ERR_ARG, "host_suite: n=%lld n_slots=%d", (long long)n, n_slots);
-    int n_out = 0;
-    if (int rc = count_outputs("host_suite", h_outs, out_mask, &n_out)) return rc;
+    void* masked[S_NSLOTS];
+    if (int rc = suite_outputs("host_suite", h_outs, out_mask, false, masked)) return rc;
     if (n == 0) return EK_OK;
     if (!aligned16(workspace)) return set_error(EK_ERR_ARG, "host_suite: workspace must be 16-byte aligned");
-    const int n_arr = 3 + n_out;
+    const int n_arr = 3 + __builtin_popcount(out_mask);
     int64_t chunk = (int64_t)(workspace_bytes / ((size_t)n_slots * n_arr * sizeof(T)));
     chunk -= chunk % 4096;  // keeps every sub-buffer 16-byte aligned and tiles whole
     if (chunk <= 0) return set_error(EK_ERR_PIPE, "host_suite: workspace of %zu bytes is too small for %d slots", workspace_bytes, n_slots);
@@ -189,14 +178,14 @@ static int host_suite_tq_hybrid(const char* what, const void* h_t, const void* h
         return set_error(EK_ERR_ENUM, "%s: invalid height mode %d", what, height_mode);
     const bool zs_row = geo && (h_cols[1] || (h_cols[2] && exactm::height_adds_zs(height_mode)));
     if (zs_row && !h_zs) return set_error(EK_ERR_ARG, "%s: this output needs the surface geopotential zs", what);
-    int n_out = 0;
-    if (int rc = count_outputs(what, h_outs, out_mask, &n_out, geo)) return rc;
+    void* masked[S_NSLOTS];
+    if (int rc = suite_outputs(what, h_outs, out_mask, geo, masked)) return rc;
     if (npl == 0) return EK_OK;
     if (!aligned16(workspace)) return set_error(EK_ERR_ARG, "%s: workspace must be 16-byte aligned", what);
     const size_t coef = (((size_t)(nlev + 1) * sizeof(T) + 255u) / 256u) * 256u;  // A, then B, at the start of the workspace
     if (workspace_bytes <= 2 * coef) return set_error(EK_ERR_PIPE, "%s: workspace of %zu bytes is too small", what, workspace_bytes);
     // device rows of one chunk: t, q, outputs, column outputs (nlev each) + sp (+ zs)
-    const int64_t rows = (int64_t)(2 + n_out + n_col) * nlev + 1 + (zs_row ? 1 : 0);
+    const int64_t rows = (int64_t)(2 + __builtin_popcount(out_mask) + n_col) * nlev + 1 + (zs_row ? 1 : 0);
     int64_t chunk = (int64_t)((workspace_bytes - 2 * coef) / ((size_t)n_slots * rows * sizeof(T)));
     chunk -= chunk % 1024;  // whole vectors, 16-byte aligned rows
     if (chunk <= 0) return set_error(EK_ERR_PIPE, "%s: workspace of %zu bytes is too small for %d slots of %d levels", what, workspace_bytes, n_slots, nlev);

@@ -524,23 +524,38 @@ __global__ void __launch_bounds__(kThreads, kGeoMinCtas) suite_geo_kernel(const 
     }
 }
 
-int grid_for(int64_t items) {
-    const int sms = sm_count_current_device();
-    if (sms <= 0) return -1;
+// one CTA per work item, at most g_ctas_per_sm per SM
+int grid_for(const char* what, int64_t items, int& blocks) {
+    int sms;
+    if (int rc = current_sms(what, sms)) return rc;
     const int64_t cap = (int64_t)sms * g_ctas_per_sm.load(std::memory_order_relaxed);
-    return (int)(items < cap ? (items > 0 ? items : 1) : cap);
+    blocks = (int)(items < cap ? (items > 0 ? items : 1) : cap);
+    return EK_OK;
 }
 
-// levels per work item: enough items to balance the grid, at least 2 levels each
-int rows_per_item_for(int64_t ptiles, int n_rows) {
-    const int sms = sm_count_current_device();
-    const int64_t want_items = (int64_t)(sms > 0 ? sms : 148) * 64;
-    int64_t chunks = (want_items + ptiles - 1) / ptiles;
+// levels per work item of a level-chunked launch over npl columns and n_rows levels: enough items to balance the grid, at least
+// 2 levels each; `items` is their number
+template <typename T> int rows_per_item_for(const char* what, int64_t npl, int n_rows, int& rows_per_item, int64_t& items) {
+    int sms;
+    if (int rc = current_sms(what, sms)) return rc;
+    constexpr int TILE = kThreads * Vec16<T>::N;
+    const int64_t ptiles = (npl + TILE - 1) / TILE;
+    int64_t chunks = ((int64_t)sms * 64 + ptiles - 1) / ptiles;
     if (chunks < 1) chunks = 1;
     int rpi = (int)((n_rows + chunks - 1) / chunks);
     if (rpi < 2) rpi = 2;
     if (rpi & 1) ++rpi;
-    return rpi;
+    rows_per_item = rpi;
+    items = ptiles * ((n_rows + rpi - 1) / rpi);
+    return EK_OK;
+}
+
+// Dynamic shared memory of a hybrid launch: the lean tables (float64) + the copy of the nlev + 1 half-level coefficients A, B
+// (none when `coefs` is false: alpha / delta given).
+template <typename T> int hybrid_smem(const char* what, int nlev, bool coefs, unsigned& smem) {
+    smem = smem_for<T>() + (coefs ? coef_smem_bytes<T>(nlev + 1) : 0u);
+    if (smem > 200u * 1024u) return set_error(EK_ERR_ARG, "%s: nlev=%d is too large for the shared-memory coefficient copy", what, nlev);
+    return EK_OK;
 }
 
 bool ok16(const void* p) { return p == nullptr || aligned16(p); }
@@ -559,22 +574,14 @@ static int impl_pressure_on_hybrid_levels(const void* A, const void* B, int nhal
     if (npl == 0) return EK_OK;
     HybridArgs g{sp, A, B, full_rows, half_rows, (full || delta || alpha) ? n_full : 0, half ? n_half : 0, top_k, top_toa, alpha_top,
                  full, half, delta, alpha, npl, 2, (alpha_delta_f64 || sizeof(T) == 8) ? 1 : 0};
-    constexpr int TILE = kThreads * Vec16<T>::N;
-    const int64_t ptiles = (npl + TILE - 1) / TILE;
-    const int n_rows = g.n_full > g.n_half ? g.n_full : g.n_half;
-    g.rows_per_item = rows_per_item_for(ptiles, n_rows);
-    const int64_t items = ptiles * ((n_rows + g.rows_per_item - 1) / g.rows_per_item);
-    const int blocks = grid_for(items);
-    if (blocks < 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
+    int64_t items;
+    int blocks;
+    if (int rc = rows_per_item_for<T>(what, npl, g.n_full > g.n_half ? g.n_full : g.n_half, g.rows_per_item, items)) return rc;
+    if (int rc = grid_for(what, items, blocks)) return rc;
     const bool vec = npl % Vec16<T>::N == 0 && ok16(sp) && ok16(full) && ok16(half) && ok16(delta) && ok16(alpha);
     const unsigned smem = (delta || alpha) ? smem_for<T>() : 0u;  // the log table, for delta / alpha only
-    const int rc = vec ? launch_kernel_smem<&hybrid_pressure_kernel<T, true>>(blocks, static_cast<cudaStream_t>(stream), smem, g)
-                       : launch_kernel_smem<&hybrid_pressure_kernel<T, false>>(blocks, static_cast<cudaStream_t>(stream), smem, g);
-    if (rc) return rc;
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
-    return EK_OK;
+    return vec ? launch_kernel_smem<&hybrid_pressure_kernel<T, true>>(what, blocks, static_cast<cudaStream_t>(stream), smem, g)
+               : launch_kernel_smem<&hybrid_pressure_kernel<T, false>>(what, blocks, static_cast<cudaStream_t>(stream), smem, g);
 }
 EK_API(pressure_on_hybrid_levels,
        (const void* A, const void* B, int nhalf, const void* sp, int64_t npl, const int* full_rows, int n_full, const int* half_rows, int n_half,
@@ -583,15 +590,13 @@ EK_API(pressure_on_hybrid_levels,
 
 template <typename T>
 static int impl_hybrid_top_is_toa(const void* sp, int64_t npl, double a_top, double b_top, int* flag, void* stream) {
-    if (!sp || !flag || npl < 0) return set_error(EK_ERR_ARG, "hybrid_top_is_toa: bad arguments");
+    const char* what = "hybrid_top_is_toa";
+    if (!sp || !flag || npl < 0) return set_error(EK_ERR_ARG, "%s: bad arguments", what);
     if (npl == 0) return EK_OK;
-    const int blocks = grid_for((npl + 255) / 256);
-    if (blocks < 0) return set_error(EK_ERR_ARG, "hybrid_top_is_toa: no CUDA device is current");
+    int blocks;
+    if (int rc = grid_for(what, (npl + 255) / 256, blocks)) return rc;
     any_le_kernel<T><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(static_cast<const T*>(sp), npl, (T)a_top, (T)b_top, (T)0.1, flag);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return set_error((int)err, "hybrid_top_is_toa: kernel launch failed: %s", cudaGetErrorString(err));
-    return EK_OK;
+    return launched(what);
 }
 EK_API(hybrid_top_is_toa, (const void* sp, int64_t npl, double a_top, double b_top, int* flag, void* stream), (sp, npl, a_top, b_top, flag, stream))
 
@@ -608,53 +613,30 @@ static int impl_geopotential_on_hybrid_levels(const void* t, const void* q, int 
     if (npl == 0) return EK_OK;
     GeoArgs g{t, q, sp, A, B, alpha, delta, zs, out, nlev, npl, given ? 0 : nhalf - 1 - nlev, top_toa, alpha_top, mode};
     constexpr int TILE = kThreads * Vec16<T>::N;
-    const int blocks = grid_for((npl + TILE - 1) / TILE);
-    if (blocks < 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
+    int blocks;
+    if (int rc = grid_for(what, (npl + TILE - 1) / TILE, blocks)) return rc;
     const bool vec = npl % Vec16<T>::N == 0 && ok16(t) && ok16(q) && ok16(sp) && ok16(alpha) && ok16(delta) && ok16(zs) && ok16(out);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const unsigned smem = smem_for<T>() + (given ? 0u : coef_smem_bytes<T>(nlev + 1));  // lean tables + the band's half-level coefficients
-    if (smem > 200u * 1024u) return set_error(EK_ERR_ARG, "%s: nlev=%d is too large for the shared-memory coefficient copy", what, nlev);
-    int rc;
+    unsigned smem;
+    if (int rc = hybrid_smem<T>(what, nlev, !given, smem)) return rc;
     if (given) {
-        if (vec) rc = launch_kernel_smem<&column_geopotential_kernel<T, true, true, -1>>(blocks, st, smem, g);
-        else rc = launch_kernel_smem<&column_geopotential_kernel<T, true, false, -1>>(blocks, st, smem, g);
-    } else if (!vec) {
-        rc = launch_kernel_smem<&column_geopotential_kernel<T, false, false, -1>>(blocks, st, smem, g);
-    } else {  // the whole-field case: one instantiation per output form
-        switch (mode) {
-            case EK_HM_THICKNESS: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_THICKNESS>>(blocks, st, smem, g); break;
-            case EK_HM_GEOPOTENTIAL: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOPOTENTIAL>>(blocks, st, smem, g); break;
-            case EK_HM_GH_SEA: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GH_SEA>>(blocks, st, smem, g); break;
-            case EK_HM_GH_GROUND: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GH_GROUND>>(blocks, st, smem, g); break;
-            case EK_HM_GEOM_SEA: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOM_SEA>>(blocks, st, smem, g); break;
-            default: rc = launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOM_GROUND>>(blocks, st, smem, g); break;
-        }
+        if (vec) return launch_kernel_smem<&column_geopotential_kernel<T, true, true, -1>>(what, blocks, st, smem, g);
+        return launch_kernel_smem<&column_geopotential_kernel<T, true, false, -1>>(what, blocks, st, smem, g);
     }
-    if (rc) return rc;
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
-    return EK_OK;
+    if (!vec) return launch_kernel_smem<&column_geopotential_kernel<T, false, false, -1>>(what, blocks, st, smem, g);
+    switch (mode) {  // the whole-field case: one instantiation per output form
+        case EK_HM_THICKNESS: return launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_THICKNESS>>(what, blocks, st, smem, g);
+        case EK_HM_GEOPOTENTIAL: return launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOPOTENTIAL>>(what, blocks, st, smem, g);
+        case EK_HM_GH_SEA: return launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GH_SEA>>(what, blocks, st, smem, g);
+        case EK_HM_GH_GROUND: return launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GH_GROUND>>(what, blocks, st, smem, g);
+        case EK_HM_GEOM_SEA: return launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOM_SEA>>(what, blocks, st, smem, g);
+        default: return launch_kernel_smem<&column_geopotential_kernel<T, false, true, EK_HM_GEOM_GROUND>>(what, blocks, st, smem, g);
+    }
 }
 EK_API(geopotential_on_hybrid_levels,
        (const void* t, const void* q, int nlev, int64_t npl, const void* sp, const void* A, const void* B, int nhalf, int top_toa,
         double alpha_top, const void* alpha, const void* delta, const void* zs, int mode, void* out, void* stream),
        (t, q, nlev, npl, sp, A, B, nhalf, top_toa, alpha_top, alpha, delta, zs, mode, out, stream))
-
-// The suite arguments shared by the hybrid launchers: the ept method (reset to IFS when no slot uses it) and the output table
-// of the requested slots; `vec` is cleared when a buffer is not 16-byte aligned.
-static int suite_outputs(const char* what, void* const* outs, uint32_t out_mask, bool any_other, int& ept_method, void** dst, bool& vec) {
-    if (out_mask >= (1u << S_NSLOTS) || (out_mask == 0 && !any_other)) return set_error(EK_ERR_ARG, "%s: out_mask=0x%x selects no output", what, out_mask);
-    constexpr uint32_t EPT = (1u << S_EPT) | (1u << S_WBPT);
-    if (!(out_mask & EPT)) ept_method = EK_EPT_IFS;
-    if (ept_method < EK_EPT_IFS || ept_method > EK_EPT_BOLTON39) return set_error(EK_ERR_ENUM, "%s: invalid ept method id %d", what, ept_method);
-    for (int k = 0; k < S_NSLOTS; ++k) {
-        dst[k] = ((out_mask >> k) & 1u) ? (outs ? outs[k] : nullptr) : nullptr;
-        if (((out_mask >> k) & 1u) && !dst[k]) return set_error(EK_ERR_ARG, "%s: output %d requested but its buffer is NULL", what, k);
-        vec = vec && ok16(dst[k]);
-    }
-    return EK_OK;
-}
 
 // The suite instantiations of the hybrid kernels: a run-time mask for each non-IFS ept method, and for IFS the two common static
 // masks (the default five outputs, and those with ept + wbpt) or a run-time mask.  LAUNCH(MASK, EPT_METHOD) launches one.
@@ -678,35 +660,25 @@ static int suite_hybrid(const void* t, const void* q, const void* sp, const void
     const char* what = "suite_tq_hybrid";
     if (!t || !q || !sp || !A || !B || nlev < 1 || npl < 0) return set_error(EK_ERR_ARG, "%s: bad arguments", what);
     SuiteHybridArgs g{t, q, sp, A, B, {}, p_out, nlev, npl, 2};
+    if (int rc = suite_outputs(what, outs, out_mask, p_out != nullptr, g.outs)) return rc;
+    if (int rc = suite_ept_method(what, out_mask, ept_method)) return rc;
     bool vec = npl % Vec16<T>::N == 0 && ok16(t) && ok16(q) && ok16(sp) && ok16(p_out);
-    if (int rc = suite_outputs(what, outs, out_mask, p_out != nullptr, ept_method, g.outs, vec)) return rc;
+    for (void* o : g.outs) vec = vec && ok16(o);
     if (npl == 0) return EK_OK;
-    constexpr int TILE = kThreads * Vec16<T>::N;
-    const int64_t ptiles = (npl + TILE - 1) / TILE;
-    g.rows_per_item = rows_per_item_for(ptiles, nlev);
-    const int64_t items = ptiles * ((nlev + g.rows_per_item - 1) / g.rows_per_item);
-    const int blocks = grid_for(items);
-    if (blocks < 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
+    int64_t items;
+    int blocks;
+    if (int rc = rows_per_item_for<T>(what, npl, nlev, g.rows_per_item, items)) return rc;
+    if (int rc = grid_for(what, items, blocks)) return rc;
     Params P;
     P.out_mask = out_mask;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const unsigned smem = smem_for<T>() + coef_smem_bytes<T>(nlev + 1);  // lean tables (float64) + the half-level coefficients
-    if (smem > 200u * 1024u) return set_error(EK_ERR_ARG, "%s: nlev=%d is too large for the shared-memory coefficient copy", what, nlev);
-#define EK_LAUNCH_SH(M, EM)                                                                                      \
-    do {                                                                                                         \
-        if (vec)                                                                                                 \
-            rc = launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(blocks, st, smem, g, P); \
-        else                                                                                                     \
-            rc = launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(blocks, st, smem, g, P); \
-    } while (0)
-    int rc;
+    unsigned smem;
+    if (int rc = hybrid_smem<T>(what, nlev, true, smem)) return rc;
+#define EK_LAUNCH_SH(M, EM)                                                                                                   \
+    return vec ? launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(what, blocks, st, smem, g, P) \
+               : launch_kernel_smem<&suite_hybrid_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(what, blocks, st, smem, g, P)
     EK_SUITE_DISPATCH(EK_LAUNCH_SH);
-    if (rc) return rc;
 #undef EK_LAUNCH_SH
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
-    return EK_OK;
 }
 
 template <template <uint32_t, int> class OpM, template <uint32_t, int> class OpME, typename T>
@@ -721,34 +693,26 @@ static int suite_hybrid_geo(const void* t, const void* q, const void* sp, const 
     if (need_zs && !zs) return set_error(EK_ERR_ARG, "%s: this output needs the surface geopotential zs", what);
     SuiteGeoArgs g{t, q, sp, need_zs ? zs : nullptr, A, B, {}, p_out, thickness_out, z_out, height_out, nlev, npl, top_toa, alpha_top,
                    height_out ? height_mode : EK_HM_THICKNESS};
+    const bool other = p_out || thickness_out || z_out || height_out;
+    if (int rc = suite_outputs(what, outs, out_mask, other, g.outs)) return rc;
+    if (int rc = suite_ept_method(what, out_mask, ept_method)) return rc;
     bool vec = npl % Vec16<T>::N == 0 && ok16(t) && ok16(q) && ok16(sp) && ok16(g.zs) && ok16(p_out) && ok16(thickness_out) && ok16(z_out) &&
                ok16(height_out);
-    const bool other = p_out || thickness_out || z_out || height_out;
-    if (int rc = suite_outputs(what, outs, out_mask, other, ept_method, g.outs, vec)) return rc;
+    for (void* o : g.outs) vec = vec && ok16(o);
     if (npl == 0) return EK_OK;
     constexpr int TILE = kThreads * Vec16<T>::N;
-    const int blocks = grid_for((npl + TILE - 1) / TILE);  // one work item per column tile: the level walk is sequential
-    if (blocks < 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
+    int blocks;
+    if (int rc = grid_for(what, (npl + TILE - 1) / TILE, blocks)) return rc;  // one work item per column tile: the level walk is sequential
     Params P;
     P.out_mask = out_mask;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const unsigned smem = smem_for<T>() + coef_smem_bytes<T>(nlev + 1);  // lean tables (float64) + the half-level coefficients
-    if (smem > 200u * 1024u) return set_error(EK_ERR_ARG, "%s: nlev=%d is too large for the shared-memory coefficient copy", what, nlev);
-#define EK_LAUNCH_SG(M, EM)                                                                                      \
-    do {                                                                                                         \
-        if (vec)                                                                                                 \
-            rc = launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(blocks, st, smem, g, P); \
-        else                                                                                                     \
-            rc = launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(blocks, st, smem, g, P); \
-    } while (0)
-    int rc;
+    unsigned smem;
+    if (int rc = hybrid_smem<T>(what, nlev, true, smem)) return rc;
+#define EK_LAUNCH_SG(M, EM)                                                                                                \
+    return vec ? launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, true>>(what, blocks, st, smem, g, P) \
+               : launch_kernel_smem<&suite_geo_kernel<OpM<M, EM>, OpME<M, EM>, T, false>>(what, blocks, st, smem, g, P)
     EK_SUITE_DISPATCH(EK_LAUNCH_SG);
-    if (rc) return rc;
 #undef EK_LAUNCH_SG
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
-    return EK_OK;
 }
 
 template <typename T>

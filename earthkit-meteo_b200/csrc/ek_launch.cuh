@@ -60,21 +60,26 @@ template <auto Kernel> inline int prepare_smem(unsigned smem_bytes) {
     return EK_OK;
 }
 
-// prepare_smem + launch of a kernel with the standard CTA size and the dtype's dynamic shared memory; nonzero: not launched
-template <auto Kernel, typename... Args> inline int launch_kernel_smem(int blocks, cudaStream_t st, unsigned smem, Args... args) {
-    if (int rc = prepare_smem<Kernel>(smem)) return rc;
-    Kernel<<<blocks, kThreads, smem, st>>>(args...);
+// Counts the launch just issued and reports its launch error, if any.
+inline int launched(const char* what) {
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
     return EK_OK;
 }
-template <auto Kernel, typename T, typename... Args> inline int launch_kernel(int blocks, cudaStream_t st, Args... args) {
-    return launch_kernel_smem<Kernel>(blocks, st, smem_for<T>(), args...);
+
+// prepare_smem + launch of a kernel with the standard CTA size and `smem` bytes of dynamic shared memory
+template <auto Kernel, typename... Args> inline int launch_kernel_smem(const char* what, int blocks, cudaStream_t st, unsigned smem, Args... args) {
+    if (int rc = prepare_smem<Kernel>(smem)) return rc;
+    Kernel<<<blocks, kThreads, smem, st>>>(args...);
+    return launched(what);
 }
 
 // Launch of a streaming kernel that orders itself behind its predecessor in the stream with pdl_acquire() (ek_thermo_kernels.cuh):
 // the programmatic-serialization attribute lets it be scheduled while the predecessor drains.  ONLY for kernels that call
 // pdl_acquire() before their first access to a field -- without it the attribute would remove the stream dependency.
 template <auto Kernel, typename... Args>
-inline int launch_streaming(unsigned blocks, unsigned smem, cudaStream_t st, Args... args) {
+inline int launch_streaming(const char* what, unsigned blocks, unsigned smem, cudaStream_t st, Args... args) {
     if (int rc = prepare_smem<Kernel>(smem)) return rc;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(blocks);
@@ -87,7 +92,28 @@ inline int launch_streaming(unsigned blocks, unsigned smem, cudaStream_t st, Arg
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     cudaLaunchKernelEx(&cfg, Kernel, args...);
+    return launched(what);
+}
+
+// The SM count of the current device; EK_ERR_ARG when no device is current.
+inline int current_sms(const char* what, int& sms) {
+    sms = sm_count_current_device();
+    if (sms <= 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
     return EK_OK;
+}
+
+// Grid of a streaming launch of Op over ntiles whole tiles plus tail_blocks CTAs' worth of remainder on `sms` SMs: at most
+// g_ctas_per_sm CTAs per SM, each walking its share of the tiles.
+template <class Op> unsigned streaming_grid(int sms, int64_t ntiles, int64_t tail_blocks) {
+    int64_t cap = (int64_t)sms * g_ctas_per_sm.load(std::memory_order_relaxed);
+    // small fields (a few tiles per resident CTA, e.g. one ERA5 level): exactly one resident wave -- every CTA copies the lean
+    // tables once and walks its 2-3 tiles back to back instead of a second, partial wave of CTAs queueing behind the first
+    // (theta + rh on 1 M points, graph replay: 14.4 -> 12.3 us; profiles/r02_kbench_era5_ctas.log)
+    const int64_t wave = (int64_t)sms * MinCtasOf<Op>::value;
+    if (ntiles <= 8 * wave && wave < cap) cap = wave;
+    int64_t blocks = ntiles > tail_blocks ? ntiles : tail_blocks;
+    if (blocks > cap) blocks = cap;
+    return blocks < 1 ? 1u : (unsigned)blocks;
 }
 
 // Launch Op over n points.  ins[k].ptr == NULL means broadcast scalar ins[k].value; outs[o] == NULL means
@@ -126,24 +152,10 @@ int launch(const char* what, const ek_operand* ins, void* const* outs, int64_t n
     const int64_t tile = (int64_t)threads * Vec16<T>::N * unroll;
     const int64_t ntiles = n / tile;
     const int64_t tail_blocks = ((n - ntiles * tile) + threads - 1) / threads;
-    const int sms = sm_count_current_device();
-    if (sms <= 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
-    int64_t cap = (int64_t)sms * g_ctas_per_sm.load(std::memory_order_relaxed);
-    // small fields (a few tiles per resident CTA, e.g. one ERA5 level): exactly one resident wave -- every CTA copies the lean
-    // tables once and walks its 2-3 tiles back to back instead of a second, partial wave of CTAs queueing behind the first
-    // (theta + rh on 1 M points, graph replay: 14.4 -> 12.3 us; profiles/r02_kbench_era5_ctas.log)
-    const int64_t wave = (int64_t)sms * MinCtasOf<Op>::value;
-    if (ntiles <= 8 * wave && wave < cap) cap = wave;
-    int64_t blocks = ntiles > tail_blocks ? ntiles : tail_blocks;
-    if (blocks > cap) blocks = cap;
-    if (blocks < 1) blocks = 1;
-
-    if (int rc = launch_streaming<&ew_kernel<Op, OpE, T, unroll>>((unsigned)blocks, smem_for<T>(), static_cast<cudaStream_t>(stream), in, out, n, P, vec_ok))
-        return rc;
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
-    return EK_OK;
+    int sms;
+    if (int rc = current_sms(what, sms)) return rc;
+    return launch_streaming<&ew_kernel<Op, OpE, T, unroll>>(what, streaming_grid<Op>(sms, ntiles, tail_blocks), smem_for<T>(),
+                                                            static_cast<cudaStream_t>(stream), in, out, n, P, vec_ok);
 }
 
 // Op over n_seg separate fields of n_per_seg points each in one launch (ew_batch_kernel).  ins[k]: host array of n_seg device
@@ -163,8 +175,8 @@ int launch_batch(const char* what, int n_seg, const void* const* const* ins, con
     if (last_scalars && ins[Op::NIN - 1]) return set_error(EK_ERR_ARG, "%s: the last input is given both as fields and as per-segment scalars", what);
     P.out_mask = out_mask;
     if (n_seg == 0 || n_per_seg == 0) return EK_OK;
-    const int sms = sm_count_current_device();
-    if (sms <= 0) return set_error(EK_ERR_ARG, "%s: no CUDA device is current", what);
+    int sms;
+    if (int rc = current_sms(what, sms)) return rc;
     constexpr int unroll = UnrollOf<Op>::value;
     const int64_t tile = (int64_t)kThreads * Vec16<T>::N * unroll;
     for (int s0 = 0; s0 < n_seg; s0 += kBatchMaxSeg) {
@@ -197,19 +209,33 @@ int launch_batch(const char* what, int n_seg, const void* const* const* ins, con
             }
         const int64_t ntiles = (n_per_seg / tile) * B.n_seg;
         const int64_t tail_blocks = ((n_per_seg % tile) * B.n_seg + kThreads - 1) / kThreads;
-        int64_t cap = (int64_t)sms * g_ctas_per_sm.load(std::memory_order_relaxed);
-        const int64_t wave = (int64_t)sms * MinCtasOf<Op>::value;
-        if (ntiles <= 8 * wave && wave < cap) cap = wave;
-        int64_t blocks = ntiles > tail_blocks ? ntiles : tail_blocks;
-        if (blocks > cap) blocks = cap;
-        if (blocks < 1) blocks = 1;
-        if (int rc = launch_streaming<&ew_batch_kernel<Op, OpE, T, unroll>>((unsigned)blocks, smem_for<T>(), static_cast<cudaStream_t>(stream), B, n_per_seg, P,
-                                                                            vec_ok))
+        if (int rc = launch_streaming<&ew_batch_kernel<Op, OpE, T, unroll>>(what, streaming_grid<Op>(sms, ntiles, tail_blocks), smem_for<T>(),
+                                                                            static_cast<cudaStream_t>(stream), B, n_per_seg, P, vec_ok))
             return rc;
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess) return set_error((int)err, "%s: kernel launch failed: %s", what, cudaGetErrorString(err));
     }
+    return EK_OK;
+}
+
+// The output table of a suite call: dst[k] = outs[k] for every slot k requested in out_mask, NULL for the others.  Rejects a
+// mask beyond the S_NSLOTS slots, an empty mask when the call writes no other output (`other_out`: a pressure or column output),
+// and a requested slot without a buffer.  E: a device pointer, or the host array of per-segment pointers of a batch call.
+template <typename E> int suite_outputs(const char* what, const E* outs, uint32_t out_mask, bool other_out, E* dst) {
+    if (out_mask >= (1u << S_NSLOTS) || (out_mask == 0 && !other_out))
+        return set_error(EK_ERR_ARG, "%s: out_mask=0x%x selects no valid output", what, out_mask);
+    if (out_mask && !outs) return set_error(EK_ERR_ARG, "%s: outs is NULL", what);
+    for (int k = 0; k < S_NSLOTS; ++k) {
+        const bool want = (out_mask >> k) & 1u;
+        dst[k] = want ? outs[k] : nullptr;
+        if (want && !dst[k]) return set_error(EK_ERR_ARG, "%s: output %d requested but its buffer is NULL", what, k);
+    }
+    return EK_OK;
+}
+
+// The ept formulation of a suite call only matters for slots 8 / 9 (ept, wbpt): reset to IFS when neither is requested, else
+// it must be one of EK_EPT_*.
+inline int suite_ept_method(const char* what, uint32_t out_mask, int& ept_method) {
+    if (!(out_mask & ((1u << S_EPT) | (1u << S_WBPT)))) ept_method = EK_EPT_IFS;
+    if (ept_method < EK_EPT_IFS || ept_method > EK_EPT_BOLTON39) return set_error(EK_ERR_ENUM, "%s: invalid ept method id %d", what, ept_method);
     return EK_OK;
 }
 

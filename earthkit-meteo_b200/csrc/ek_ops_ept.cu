@@ -19,15 +19,12 @@ __global__ void bisect_tab_init_kernel() {
     }
 #endif
 }
-static int bisect_prepare(void* stream) {
+static int bisect_prepare(const char* what, void* stream) {
     bisect_tab_init_kernel<<<16, 256, kSmemBytes, static_cast<cudaStream_t>(stream)>>>();
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return set_error((int)err, "bisect table init failed: %s", cudaGetErrorString(err));
-    return EK_OK;
+    return launched(what);
 }
 #else
-static int bisect_prepare(void*) { return EK_OK; }
+static int bisect_prepare(const char*, void*) { return EK_OK; }
 #endif
 
 template <typename T, int M, int TM, int HUM = -1>
@@ -38,7 +35,7 @@ static int ept_wb_mt(ek_operand t, ek_operand h, ek_operand p, int hum, int at_p
     P.opt0 = hum;
     P.opt1 = at_p0;
     if (TM == TM_BISECT && n > 0) {
-        const int rc = bisect_prepare(stream);
+        const int rc = bisect_prepare("ept_wet_bulb", stream);
         if (rc != EK_OK) return rc;
     }
     return launch<EK_OPS(OpEptWb<M, TM, HUM>), T>("ept_wet_bulb", ins, outs, n, P, stream);
@@ -118,7 +115,7 @@ EK_API(saturation_ept, (ek_operand t, ek_operand p, int m, void* out, int64_t n,
 template <typename T, int M> static int t_on_ma_m(int tm, const ek_operand* ins, void* const* outs, int64_t n, void* stream) {
     if (tm == EK_TM_BISECT) {
         if (n > 0) {
-            const int rc = bisect_prepare(stream);
+            const int rc = bisect_prepare("temperature_on_moist_adiabat", stream);
             if (rc != EK_OK) return rc;
         }
         return launch<EK_OPS(OpTOnMa<M, TM_BISECT>), T>("temperature_on_moist_adiabat", ins, outs, n, Params{}, stream);

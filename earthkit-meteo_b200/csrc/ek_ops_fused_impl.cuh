@@ -8,16 +8,10 @@ using namespace ek;
 template <template <uint32_t, int> class OpM, template <uint32_t, int> class OpME, typename T>
 static int suite(const char* what, ek_operand a, ek_operand b, ek_operand c, void* const* outs, uint32_t out_mask, int ept_method, int64_t n,
                  void* stream) {
-    if (!outs) return set_error(EK_ERR_ARG, "%s: outs is NULL", what);
-    if (out_mask == 0 || out_mask >= (1u << S_NSLOTS)) return set_error(EK_ERR_ARG, "%s: out_mask=0x%x selects no valid output", what, out_mask);
     void* o[S_NSLOTS];
-    for (int k = 0; k < S_NSLOTS; ++k) {
-        o[k] = (out_mask >> k) & 1u ? outs[k] : nullptr;
-        if (((out_mask >> k) & 1u) && !outs[k]) return set_error(EK_ERR_ARG, "%s: output %d requested but its buffer is NULL", what, k);
-    }
+    if (int rc = suite_outputs(what, outs, out_mask, false, o)) return rc;
+    if (int rc = suite_ept_method(what, out_mask, ept_method)) return rc;
     ek_operand ins[3] = {a, b, c};
-    constexpr uint32_t EPT = (1u << S_EPT) | (1u << S_WBPT);
-    if (!(out_mask & EPT)) ept_method = EK_EPT_IFS;  // the formulation only matters for slots 8 / 9
     // output sets with a dedicated compile-time instantiation (the bench / config workloads); any other set
     // runs the generic kernel that tests the mask at run time
     switch (ept_method) {
@@ -32,9 +26,8 @@ static int suite(const char* what, ek_operand a, ek_operand b, ek_operand c, voi
                 default: return launch<OpM<0, EPT_IFS>, OpME<0, EPT_IFS>, T>(what, ins, o, n, Params{}, stream);
             }
         case EK_EPT_BOLTON35: return launch<OpM<0, EPT_BOLTON35>, OpME<0, EPT_BOLTON35>, T>(what, ins, o, n, Params{}, stream);
-        case EK_EPT_BOLTON39: return launch<OpM<0, EPT_BOLTON39>, OpME<0, EPT_BOLTON39>, T>(what, ins, o, n, Params{}, stream);
+        default: return launch<OpM<0, EPT_BOLTON39>, OpME<0, EPT_BOLTON39>, T>(what, ins, o, n, Params{}, stream);  // EK_EPT_BOLTON39
     }
-    return set_error(EK_ERR_ENUM, "%s: invalid ept method id %d", what, ept_method);
 }
 
 // The same suites over n_seg separate fields (one allocation per level / member) in one launch.  Run-time mask kernel per ept
@@ -42,16 +35,10 @@ static int suite(const char* what, ek_operand a, ek_operand b, ek_operand c, voi
 template <template <uint32_t, int> class OpM, template <uint32_t, int> class OpME, typename T>
 static int suite_batch(const char* what, int n_seg, const void* const* a, const void* const* b, const void* const* c, const double* scalars,
                        const double* level_scalars, void* const* const* outs, uint32_t out_mask, int ept_method, int64_t n_per_seg, void* stream) {
-    if (!outs) return set_error(EK_ERR_ARG, "%s: outs is NULL", what);
-    if (out_mask == 0 || out_mask >= (1u << S_NSLOTS)) return set_error(EK_ERR_ARG, "%s: out_mask=0x%x selects no valid output", what, out_mask);
     void* const* o[S_NSLOTS];
-    for (int k = 0; k < S_NSLOTS; ++k) {
-        o[k] = (out_mask >> k) & 1u ? outs[k] : nullptr;
-        if (((out_mask >> k) & 1u) && !outs[k]) return set_error(EK_ERR_ARG, "%s: output %d requested but its pointer array is NULL", what, k);
-    }
+    if (int rc = suite_outputs(what, outs, out_mask, false, o)) return rc;
+    if (int rc = suite_ept_method(what, out_mask, ept_method)) return rc;
     const void* const* ins[3] = {a, b, c};
-    constexpr uint32_t EPT = (1u << S_EPT) | (1u << S_WBPT);
-    if (!(out_mask & EPT)) ept_method = EK_EPT_IFS;
     switch (ept_method) {
         case EK_EPT_IFS:
             switch (out_mask) {
@@ -61,7 +48,6 @@ static int suite_batch(const char* what, int n_seg, const void* const* a, const 
                 default: return launch_batch<OpM<0, EPT_IFS>, OpME<0, EPT_IFS>, T>(what, n_seg, ins, scalars, level_scalars, o, n_per_seg, Params{}, stream);
             }
         case EK_EPT_BOLTON35: return launch_batch<OpM<0, EPT_BOLTON35>, OpME<0, EPT_BOLTON35>, T>(what, n_seg, ins, scalars, level_scalars, o, n_per_seg, Params{}, stream);
-        case EK_EPT_BOLTON39: return launch_batch<OpM<0, EPT_BOLTON39>, OpME<0, EPT_BOLTON39>, T>(what, n_seg, ins, scalars, level_scalars, o, n_per_seg, Params{}, stream);
+        default: return launch_batch<OpM<0, EPT_BOLTON39>, OpME<0, EPT_BOLTON39>, T>(what, n_seg, ins, scalars, level_scalars, o, n_per_seg, Params{}, stream);  // EK_EPT_BOLTON39
     }
-    return set_error(EK_ERR_ENUM, "%s: invalid ept method id %d", what, ept_method);
 }
