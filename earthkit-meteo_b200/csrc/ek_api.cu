@@ -69,6 +69,7 @@ extern "C" EK_EXPORT int ek_thermo_shard_range(int64_t n, int world, int rank, i
 // defined in ek_ops_fused_*.cu / ek_hybrid.cu (so the suite kernels are instantiated in one translation unit only)
 template <typename T> int ek_suite_launch_tqp(const ek_operand* ins, void* const* outs, uint32_t mask, int ept_method, int64_t n, void* stream);
 template <typename T> int ek_suite_launch_ttdp(const ek_operand* ins, void* const* outs, uint32_t mask, int ept_method, int64_t n, void* stream);
+template <typename T> int ek_suite_launch_trp(const ek_operand* ins, void* const* outs, uint32_t mask, int ept_method, int64_t n, void* stream);
 template <typename T>
 int ek_suite_launch_hybrid(const void* t, const void* q, const void* sp, const void* A, const void* B, int nlev, int64_t npl, void* const* outs,
                            uint32_t out_mask, int ept_method, void* stream);
@@ -110,7 +111,7 @@ struct StreamSet {
 template <typename T>
 static int impl_host_suite(int kind, const void* h_a, const void* h_b, const void* h_c, void* const* h_outs, uint32_t out_mask, int ept_method,
                            int64_t n, void* workspace, size_t workspace_bytes, int n_slots) {
-    if (kind != 0 && kind != 1) return set_error(EK_ERR_ENUM, "host_suite: kind=%d", kind);
+    if (kind < 0 || kind > 2) return set_error(EK_ERR_ENUM, "host_suite: kind=%d", kind);
     if (!h_a || !h_b || !h_c || !h_outs || !workspace) return set_error(EK_ERR_ARG, "host_suite: NULL buffer");
     if (n < 0 || n_slots < 1 || n_slots > 16) return set_error(EK_ERR_ARG, "host_suite: n=%lld n_slots=%d", (long long)n, n_slots);
     void* masked[S_NSLOTS];
@@ -144,7 +145,9 @@ static int impl_host_suite(int kind, const void* h_a, const void* h_b, const voi
         void* douts[S_NSLOTS];
         int j = 0;
         for (int k = 0; k < S_NSLOTS; ++k) douts[k] = ((out_mask >> k) & 1u) ? (void*)(base + (int64_t)(3 + j++) * chunk) : nullptr;
-        int rc = kind == 0 ? ek_suite_launch_tqp<T>(ins, douts, out_mask, ept_method, m, st) : ek_suite_launch_ttdp<T>(ins, douts, out_mask, ept_method, m, st);
+        int rc = kind == 0   ? ek_suite_launch_tqp<T>(ins, douts, out_mask, ept_method, m, st)
+                 : kind == 1 ? ek_suite_launch_ttdp<T>(ins, douts, out_mask, ept_method, m, st)
+                             : ek_suite_launch_trp<T>(ins, douts, out_mask, ept_method, m, st);
         if (rc != EK_OK) return rc;
         for (int k = 0; k < S_NSLOTS; ++k)
             if (douts[k]) {

@@ -1,5 +1,5 @@
-// ek_ops_fused_impl.cuh -- fused multi-output suites: read (t,q,p) or (t,td,p) once, write every requested field.
-// Included by ek_ops_fused_tqp.cu / ek_ops_fused_ttdp.cu (one translation unit per suite, compiled in parallel).
+// ek_ops_fused_impl.cuh -- fused multi-output suites: read (t,q,p), (t,td,p) or (t,r,p) once, write every requested field.
+// Included by ek_ops_fused_tqp.cu / ek_ops_fused_ttdp.cu / ek_ops_fused_trp.cu (one translation unit per suite, compiled in parallel).
 #pragma once
 #include "ek_launch.cuh"
 

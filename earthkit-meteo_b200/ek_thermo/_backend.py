@@ -103,12 +103,12 @@ for _name, (_nin, _opts, _nout) in SIGNATURES.items():
         _fn = getattr(_lib, f"ek_thermo_{_name}_{_sfx}")
         _fn.argtypes = [ek_operand] * _nin + list(_opts) + [c_void_p] * _nout + [c_int64, c_void_p]
         _fn.restype = c_int
-for _name in ("suite_tqp", "suite_ttdp"):
+for _name in ("suite_tqp", "suite_ttdp", "suite_trp"):
     for _sfx in ("f64", "f32"):
         _fn = getattr(_lib, f"ek_thermo_{_name}_{_sfx}")
         _fn.argtypes = [ek_operand] * 3 + [ctypes.POINTER(c_void_p), c_uint32, c_int, c_int64, c_void_p]
         _fn.restype = c_int
-for _name in ("suite_tqp_batch", "suite_ttdp_batch"):
+for _name in ("suite_tqp_batch", "suite_ttdp_batch", "suite_trp_batch"):
     for _sfx in ("f64", "f32"):
         _fn = getattr(_lib, f"ek_thermo_{_name}_{_sfx}")
         _fn.argtypes = [c_int, c_void_p, c_void_p, c_void_p, ctypes.POINTER(c_double), ctypes.POINTER(c_double), ctypes.POINTER(c_void_p), c_uint32, c_int,

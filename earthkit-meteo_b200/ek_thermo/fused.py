@@ -1,8 +1,8 @@
 """Fused multi-output kernels: read the state of each grid point once, write every requested field.
 
 These have no counterpart function in the reference; every output equals the reference function
-named in ``SUITE_TQP_OUTPUTS`` / ``SUITE_TTDP_OUTPUTS`` applied to the same inputs (the oracle's
-``suite_tqp`` / ``suite_ttdp`` state that composition).  HBM traffic per point is
+named in ``SUITE_TQP_OUTPUTS`` / ``SUITE_TTDP_OUTPUTS`` / ``SUITE_TRP_OUTPUTS`` applied to the same inputs (the
+oracle's ``suite_tqp`` / ``suite_ttdp`` and the tests' ``trp_parity.suite_trp`` state that composition).  HBM traffic per point is
 ``8 * (3 + len(outputs))`` bytes in float64, instead of one full read+write pass per function.
 """
 from __future__ import annotations
@@ -41,6 +41,20 @@ SUITE_TTDP_OUTPUTS = {
     "ept": 8,  # ept_from_dewpoint(t, td, p, method=ept_method)          T:1326-1387
     "wbpt": 9,  # wet_bulb_potential_temperature_from_dewpoint(t, td, p, ept_method, t_method="direct")  T:1593-1634
 }
+# q = specific_humidity_from_relative_humidity(t, r, p) (T:629-663), r in %; "ept" / "wbpt" follow q, so their dewpoint is
+# dewpoint_from_specific_humidity(q, p) (T:1036-1037), not the "td" slot's, which is over water and differs below T0
+SUITE_TRP_OUTPUTS = {
+    "theta": 0,  # potential_temperature(t, p)
+    "es": 1,  # saturation_vapour_pressure(t)
+    "td": 2,  # dewpoint_from_relative_humidity(t, r)                    T:666-699
+    "q": 3,  # specific_humidity_from_relative_humidity(t, r, p)         T:629-663
+    "tv": 4,  # virtual_temperature(t, q)
+    "w": 5,  # mixing_ratio_from_specific_humidity(q)
+    "e": 6,  # r * saturation_vapour_pressure(t) / 100.0                 T:662
+    "thetav": 7,  # virtual_potential_temperature(t, q, p)
+    "ept": 8,  # ept_from_specific_humidity(t, q, p, method=ept_method)
+    "wbpt": 9,  # wet_bulb_potential_temperature_from_specific_humidity(t, q, p, ept_method, t_method="direct")
+}
 # the single pass BASELINE.json names: "read t/q/p (or t/td/p) once and write theta, rh, td, theta_e and wbpt"
 SINGLE_PASS_TQP = ("theta", "rh", "td", "ept", "wbpt")
 SINGLE_PASS_TTDP = ("theta", "rh", "q", "ept", "wbpt")
@@ -49,6 +63,8 @@ ALL7_TQP = ("theta", "es", "rh", "td", "tv", "ept", "wbpt")
 ALL7_TTDP = ("theta", "es", "rh", "q", "tv", "ept", "wbpt")
 DEFAULT_TQP = ("theta", "es", "rh", "td", "tv")
 DEFAULT_TTDP = ("theta", "es", "rh", "q", "tv")
+DEFAULT_TRP = ("theta", "es", "td", "q", "tv")
+SINGLE_PASS_TRP = ("theta", "td", "q", "ept", "wbpt")
 
 _TM = {None: 0, "none": 0, "direct": 1, "bisect": 2, "newton": 3}
 
@@ -78,6 +94,14 @@ def suite_ttdp(t, td, p, outputs=DEFAULT_TTDP, out=None, ept_method="ifs"):
     return _b.execute_suite("suite_ttdp", (t, td, p), outputs, _slots(SUITE_TTDP_OUTPUTS, outputs), out, _ept_id(ept_method))
 
 
+def suite_trp(t, r, p, outputs=DEFAULT_TRP, out=None, ept_method="ifs"):
+    """One pass over (t, r, p), ``r`` the relative humidity in %, producing the requested fields; returns ``{name: tensor}``.
+
+    Each output is the reference chain named in ``SUITE_TRP_OUTPUTS``.  ``r = 0`` gives ``td = NaN``, as in the reference."""
+    outputs = tuple(outputs)
+    return _b.execute_suite("suite_trp", (t, r, p), outputs, _slots(SUITE_TRP_OUTPUTS, outputs), out, _ept_id(ept_method))
+
+
 def suite_tqp_batch(ts, qs, ps, outputs=DEFAULT_TQP, out=None, ept_method="ifs"):
     """``suite_tqp`` over a LIST of separate fields (one tensor per level / member, each its own allocation) in one launch.
 
@@ -94,6 +118,12 @@ def suite_ttdp_batch(ts, tds, ps, outputs=DEFAULT_TTDP, out=None, ept_method="if
     """``suite_ttdp`` over a list of separate fields in one launch (see ``suite_tqp_batch``)."""
     outputs = tuple(outputs)
     return _b.execute_suite_batch("suite_ttdp_batch", (ts, tds, ps), outputs, _slots(SUITE_TTDP_OUTPUTS, outputs), out, _ept_id(ept_method))
+
+
+def suite_trp_batch(ts, rs, ps, outputs=DEFAULT_TRP, out=None, ept_method="ifs"):
+    """``suite_trp`` over a list of separate fields in one launch (see ``suite_tqp_batch``)."""
+    outputs = tuple(outputs)
+    return _b.execute_suite_batch("suite_trp_batch", (ts, rs, ps), outputs, _slots(SUITE_TRP_OUTPUTS, outputs), out, _ept_id(ept_method))
 
 
 # Fields of fewer columns than this run a mixed call as the suite launch plus one geopotential_on_hybrid_levels launch per column

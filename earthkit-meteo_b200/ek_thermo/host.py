@@ -364,6 +364,10 @@ class _HostFused:
         """``fused.suite_ttdp`` for numpy arrays: returns ``{name: numpy array}``."""
         return self._suite(_fused.suite_ttdp, t, td, p, outputs, ept_method)
 
+    def suite_trp(self, t, r, p, outputs=_fused.DEFAULT_TRP, ept_method="ifs"):
+        """``fused.suite_trp`` for numpy arrays: returns ``{name: numpy array}``."""
+        return self._suite(_fused.suite_trp, t, r, p, outputs, ept_method)
+
     def ept_wet_bulb(self, t, h, p, humidity="q", ept_method="ifs", t_method="direct", potential=True):
         """``fused.ept_wet_bulb`` for numpy arrays: returns ``(ept, wet_bulb)`` as numpy arrays."""
         return _run(lambda x, y, z: _fused.ept_wet_bulb(x, y, z, humidity=humidity, ept_method=ept_method, t_method=t_method, potential=potential),

@@ -13,7 +13,7 @@ import torch
 
 from . import _backend as _b
 from ._backend import _EPT, _TORCH
-from .fused import DEFAULT_TQP, DEFAULT_TTDP, SUITE_TQP_OUTPUTS, SUITE_TTDP_OUTPUTS
+from .fused import DEFAULT_TQP, DEFAULT_TRP, DEFAULT_TTDP, SUITE_TQP_OUTPUTS, SUITE_TRP_OUTPUTS, SUITE_TTDP_OUTPUTS
 from .vertical import COLUMN_OUTPUTS, _alpha_top_value, _split_suite_outputs, _top_is_toa
 
 
@@ -97,6 +97,9 @@ class HostSuite:
 
     def suite_ttdp(self, t, td, p, outputs=DEFAULT_TTDP, out=None, ept_method="ifs"):
         return self._run(1, SUITE_TTDP_OUTPUTS, t, td, p, tuple(outputs), out, ept_method)
+
+    def suite_trp(self, t, r, p, outputs=DEFAULT_TRP, out=None, ept_method="ifs"):
+        return self._run(2, SUITE_TRP_OUTPUTS, t, r, p, tuple(outputs), out, ept_method)
 
     def suite_tq_hybrid(self, t, q, sp, A, B, outputs=DEFAULT_TQP, out=None, ept_method="ifs", zs=None, alpha_top="ifs", h_type="geometric",
                         h_reference="ground"):

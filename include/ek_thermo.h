@@ -30,7 +30,8 @@
 extern "C" {
 #endif
 
-#define EK_THERMO_VERSION 112 /* 0.1.2: the hybrid-level suite with geopotential / height of the same levels in one pass
+#define EK_THERMO_VERSION 113 /* 0.1.3: the (t, r, p) suite (suite_trp, suite_trp_batch, host_suite kind 2).
+                                  0.1.2: the hybrid-level suite with geopotential / height of the same levels in one pass
                                   (suite_tq_hybrid_geo, host_suite_tq_hybrid_geo).  0.1.1: suite slots 8 (ept) / 9 (wbpt) and their
                                   ept_method argument; host pipelines for every suite; batched suites with one pressure per level */
 
@@ -55,6 +56,12 @@ enum {
     EK_S_WBPT = 9, /* wet_bulb_potential_temperature_from_*, t_method="direct" (the reference's default), T:1637-1675 / T:1593-1634 */
     EK_S_NSLOTS = 10
 };
+/* The (t, r, p) suite uses the same slots with q = specific_humidity_from_relative_humidity(t, r, p) (T:629-663):
+ *   0 theta, 1 es, 4 tv, 5 w, 7 thetav, 8 ept, 9 wbpt   as in the (t, q, p) suite, from that q (so slots 8 / 9 use the dewpoint
+ *                                                        of q, T:1036-1037, not slot 2);
+ *   2 (EK_S_RH)      td: dewpoint_from_relative_humidity(t, r), T:666-699 (es over water);
+ *   3 (EK_S_TD_OR_Q) q;
+ *   6 (EK_S_E)       e = r * saturation_vapour_pressure(t) / 100, the vapour pressure T:662 forms on the way to q. */
 
 /* declares ek_thermo_<name>_f64 and ek_thermo_<name>_f32 with the same parameter list */
 #define EK_THERMO_FN(name, ...)              \
@@ -142,6 +149,10 @@ EK_THERMO_FN(suite_tqp, ek_operand t, ek_operand q, ek_operand p, void* const* o
 /* (t, td, p) -> any subset of {theta, es, rh, q, tv, w, e, thetav, ept, wbpt} */
 EK_THERMO_FN(suite_ttdp, ek_operand t, ek_operand td, ek_operand p, void* const* outs, uint32_t out_mask, int ept_method, int64_t n,
              void* stream)
+/* (t, r, p) -> any subset of {theta, es, td, q, tv, w, e, thetav, ept, wbpt}; r is the relative humidity in %.  Mask 0x30D is the
+ * single pass theta, td, q, theta_e, theta_w. */
+EK_THERMO_FN(suite_trp, ek_operand t, ek_operand r, ek_operand p, void* const* outs, uint32_t out_mask, int ept_method, int64_t n,
+             void* stream)
 /* The suites over n_seg SEPARATE fields of n_per_seg points each (one allocation per level / member, as a per-level caller
  * holds them) in ONE launch: a launch per 1 M-point level is latency-bound (12-16 us for 6 us of HBM time).  t / h / p: HOST
  * arrays of n_seg DEVICE pointers, or NULL for the broadcast scalar scalars[k] (k = 0, 1, 2); outs[k]: HOST array of n_seg
@@ -152,6 +163,8 @@ EK_THERMO_FN(suite_ttdp, ek_operand t, ek_operand td, ek_operand p, void* const*
 EK_THERMO_FN(suite_tqp_batch, int n_seg, const void* const* t, const void* const* q, const void* const* p, const double* scalars,
              const double* level_scalars, void* const* const* outs, uint32_t out_mask, int ept_method, int64_t n_per_seg, void* stream)
 EK_THERMO_FN(suite_ttdp_batch, int n_seg, const void* const* t, const void* const* td, const void* const* p, const double* scalars,
+             const double* level_scalars, void* const* const* outs, uint32_t out_mask, int ept_method, int64_t n_per_seg, void* stream)
+EK_THERMO_FN(suite_trp_batch, int n_seg, const void* const* t, const void* const* r, const void* const* p, const double* scalars,
              const double* level_scalars, void* const* const* outs, uint32_t out_mask, int ept_method, int64_t n_per_seg, void* stream)
 /* (t, h, p) -> ept and/or the wet-bulb (potential) temperature in one pass.  h is td or q (humidity_kind),
  * at_p0 = 1 gives the wet-bulb POTENTIAL temperature; either output pointer may be NULL (but not both);
@@ -221,7 +234,7 @@ EK_THERMO_FN(suite_tq_hybrid_geo, const void* t, const void* q, const void* sp, 
  * `n_slots` internal streams.  Host buffers should be page-locked for full PCIe speed.  `workspace` is a
  * caller-owned DEVICE buffer of workspace_bytes with no work pending on it; chunk size = workspace_bytes /
  * (n_slots * (3 + popcount(mask)) * sizeof(T)).  Block until every output byte is in host memory (also on error:
- * the pipeline's streams are drained before the call returns).  kind: 0 = suite_tqp, 1 = suite_ttdp; out_mask,
+ * the pipeline's streams are drained before the call returns).  kind: 0 = suite_tqp, 1 = suite_ttdp, 2 = suite_trp; out_mask,
  * ept_method as for the suites (slots 8 / 9 included, so the ept / wet-bulb workload has a host path too). */
 EK_THERMO_FN(host_suite, int kind, const void* h_a, const void* h_b, const void* h_c, void* const* h_outs, uint32_t out_mask,
              int ept_method, int64_t n, void* workspace, size_t workspace_bytes, int n_slots)
